@@ -5,6 +5,7 @@ bench.py -- REPET separation throughput on B200 (BASELINE.json metric).
     python bench.py [--gpus N] [--steps K] [--warmup W]            # this repo's CUDA path
     python bench.py --impl reference [--gpus N] [--steps K] ...     # the reference on the host cores
     python bench.py --probe-host-link [--gpus N]                    # copy-only ceiling of the host<->device links
+    python bench.py --steps K --dump-outputs DIR                    # also write what the last timed step computed
 
 Workload (BASELINE.json configs[1]): `repet.original` on a batch of synthetic 30 s stereo
 44.1 kHz clips, 512 clips per GPU (4096 over 8 GPUs; weak scaling, clips are independent, no
@@ -71,7 +72,14 @@ def parse_args():
     ap.add_argument("--no-numa-bind", action="store_true", help="do not bind the rank to the GPU's NUMA-local CPUs")
     ap.add_argument("--workspace-mb", type=int, default=0, help="per-chunk workspace cap of the library (0 = default)")
     ap.add_argument("--tune", default="", help="comma separated knob=value pairs for repet_set_tuning (experiments)")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "b200" or args.probe_host_link):
+        ap.error("--dump-outputs writes the outputs of the CUDA arm's separation")
+    return args
 
 
 # --------------------------------------------------------------------------------------------
@@ -608,6 +616,49 @@ def run_configs(args, torch, repet, handle, stream, device, wanted, peaks):
 # --------------------------------------------------------------------------------------------
 # the CUDA arm
 # --------------------------------------------------------------------------------------------
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_positions(number_clips, number_channels, number_samples):
+    """The sample positions dump_outputs writes for `number_clips` clips over all ranks: a fixed seeded draw, as
+    many as keep its four files within DUMP_LIMIT_BYTES."""
+    fixed = number_clips * 8 + number_channels * number_samples * 4 + 4 * 4096  # periods, clip 0, four .npy headers
+    count = (DUMP_LIMIT_BYTES - fixed) // (number_clips * number_channels * 4 + 8)
+    count = max(1, min(number_samples, count))
+    return np.sort(np.random.default_rng(0).choice(number_samples, size=count, replace=False))
+
+
+def write_dump(directory, periods, background_clip0, background_sample, positions):
+    os.makedirs(directory, exist_ok=True)
+    for name, array in (("periods", periods.astype(np.float64)), ("background_clip0", background_clip0),
+                        ("background_sample", background_sample),
+                        ("background_sample_positions", positions.astype(np.float64))):
+        np.save(os.path.join(directory, name + ".npy"), array)
+
+
+def dump_outputs(directory, torch, dist, world, rank, out_dev, periods_dev):
+    """Write what the timed path returned in its last step, so that two builds can be compared output for output
+    on the same seeded clips.  The whole background of all ranks is GBs, so rank 0 gathers and writes, in at most
+    64 MB for the whole run (every rank must call this):
+      periods                       (N,) float64, the repeating period of each of the N clips, in frames
+      background_clip0              (C, S) float32, the whole background of clip 0
+      background_sample             (N, C, K) float32, every clip's background at K sample positions
+      background_sample_positions   (K,) float64, those positions: a fixed seeded draw, the same on every run"""
+    B, C, S = out_dev.shape
+    positions = dump_positions(world * B, C, S)
+    periods = periods_dev.to(torch.float64)
+    sample = out_dev.index_select(2, torch.from_numpy(positions).to(out_dev.device))
+    if world > 1:
+        def gathered(part):
+            parts = [torch.empty_like(part) for _ in range(world)]
+            dist.all_gather(parts, part)
+            return torch.cat(parts)
+
+        periods, sample = gathered(periods), gathered(sample)
+    if rank == 0:
+        write_dump(directory, periods.cpu().numpy(), out_dev[0].cpu().numpy(), sample.cpu().numpy(), positions)
+
+
 def run_b200_arm(args, rank, local_rank, world):
     import repet_synth
 
@@ -682,6 +733,8 @@ def run_b200_arm(args, rank, local_rank, world):
     profile = handle.profile_read(reset=True)
     handle.set_profiling(False)
     periods_first = periods_dev.cpu().numpy().copy()
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, torch, dist, world, rank, out_dev, periods_dev)
 
     # ---- end to end through the public API: page-locked host arrays in and out --------------------
     host_in = pinned_in.numpy()

@@ -212,3 +212,34 @@ def test_bench_line_contract(repet):
     assert line["e2e_pcm16"]["h2d_bytes_per_step"] * 2 == line["e2e"]["h2d_bytes_per_step"]
     assert line["configs"]["cfg1"]["period"] == 286
     assert "workload" in line["config"] and "model" not in line["config"]
+
+
+def test_bench_dump_outputs(repet, tmp_path):
+    """bench.py --dump-outputs: float .npy files of at most 64 MB in all that hold what the last of the --steps timed
+    steps returned, with the backgrounds sampled at fewer positions than a clip has.  They are compared with the same
+    seeded clips through repet.separate_batch: a check of the dump, not of parity (the golden tests cover that)."""
+    import json
+    import os
+    import subprocess
+    import sys
+
+    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+    clips, steps = 8, 3
+    out = subprocess.run([sys.executable, os.path.join(root, "bench.py"), "--clips-per-gpu", str(clips), "--steps", str(steps),
+                          "--warmup", "1", "--configs", "none", "--no-e2e", "--no-cpu-baseline", "--dump-outputs", str(tmp_path)],
+                         capture_output=True, text=True, timeout=900)
+    assert out.returncode == 0, out.stderr[-3000:]
+    line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
+    assert line["steps"] == steps and line["gpu_launches"] == 7 * steps
+    files = sorted(tmp_path.glob("*.npy"))
+    assert sum(f.stat().st_size for f in files) <= 64 << 20
+    dumped = {f.stem: np.load(f) for f in files}
+    assert set(dumped) == {"periods", "background_clip0", "background_sample", "background_sample_positions"}
+    assert all(a.dtype in (np.float32, np.float64) for a in dumped.values())
+    audio = repet_synth.make_batch(0, clips, 30 * FS)
+    background, ints = repet._host.separate_batch("original", audio, FS, repet._tunables())
+    assert np.array_equal(dumped["periods"], ints[:, 0])
+    assert np.array_equal(dumped["background_clip0"], background[0])
+    positions = dumped["background_sample_positions"].astype(np.int64)
+    assert len(positions) < 30 * FS
+    assert np.array_equal(dumped["background_sample"], background[:, :, positions])

@@ -179,11 +179,63 @@ def test_bench_reference_arm_prints_the_contract_line():
     line = json.loads([l for l in out.stdout.splitlines() if l.startswith("{")][-1])
     assert line["impl"] == "reference" and line["unit"] == "audio-s/s" and line["higher_is_better"] is True
     assert line["value"] > 0 and line["n_gpus"] == 1 and line["steps"] == 1
-    # the unmodified repet.py where /root/reference exists (this container), the oracle port elsewhere (the GPU box)
-    expected_kind = "reference" if os.path.isfile("/root/reference/repet.py") else "port"
+    # the unmodified repet.py where the reference shim finds it, the oracle port everywhere else
+    import reference_shim
+
+    expected_kind = "reference" if reference_shim.available() else "port"
     assert line["cpu_baseline"]["kind"] == expected_kind and line["cpu_baseline"]["cores"] >= 1
     assert line["e2e"] == {"value": line["value"], "unit": "audio-s/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0}
     assert "workload" in line["config"] and "model" not in line["config"]
+
+
+@pytest.mark.parametrize("world", [1, 8])
+def test_bench_dump_stays_within_64_mb(tmp_path, world):
+    """bench.py --dump-outputs at 512 clips per GPU writes one set of files for the whole run, within 64 MB however
+    many GPUs share it, with the backgrounds sampled at fewer positions than a clip has."""
+    import bench
+
+    clips, channels, samples = 512 * world, bench.CHANNELS, bench.CLIP_SAMPLES
+    positions = bench.dump_positions(clips, channels, samples)
+    assert 1 <= len(positions) < samples and np.all(np.diff(positions) > 0) and positions[-1] < samples
+    bench.write_dump(str(tmp_path), np.zeros(clips, np.int32), np.zeros((channels, samples), np.float32),
+                     np.zeros((clips, channels, len(positions)), np.float32), positions)
+    assert sum(f.stat().st_size for f in tmp_path.iterdir()) <= 64 << 20
+
+
+_DUMP_WORKER = r"""
+import sys
+sys.path.insert(0, {root!r})
+import torch, torch.distributed as dist
+import bench
+dist.init_process_group("gloo")
+rank, world = dist.get_rank(), dist.get_world_size()
+out = torch.arange(3 * 2 * 5000, dtype=torch.float32).reshape(3, 2, 5000) + 1e5 * rank
+periods = torch.arange(3, dtype=torch.int32) + 10 * rank
+bench.dump_outputs({directory!r}, torch, dist, world, rank, out, periods)
+dist.destroy_process_group()
+"""
+
+
+def test_bench_dump_gathers_every_rank(tmp_path):
+    """world_size 2 on CPU: rank 0 writes the clips of both ranks in rank order, once."""
+    import bench
+
+    script = tmp_path / "worker.py"
+    directory = tmp_path / "dump"
+    script.write_text(_DUMP_WORKER.format(root=ROOT, directory=str(directory)))
+    out = subprocess.run([sys.executable, "-m", "torch.distributed.run", "--standalone", "--nproc-per-node=2", str(script)],
+                         capture_output=True, text=True, env=dict(os.environ, OMP_NUM_THREADS="1"), timeout=300)
+    assert out.returncode == 0, out.stderr[-2000:]
+    assert sorted(f.name for f in directory.iterdir()) == [
+        "background_clip0.npy", "background_sample.npy", "background_sample_positions.npy", "periods.npy"]
+    dumped = {name: np.load(directory / (name + ".npy")) for name in ("periods", "background_clip0", "background_sample",
+                                                                      "background_sample_positions")}
+    outputs = [np.arange(3 * 2 * 5000, dtype=np.float32).reshape(3, 2, 5000) + 1e5 * rank for rank in range(2)]
+    positions = bench.dump_positions(6, 2, 5000)
+    assert np.array_equal(dumped["periods"], [0, 1, 2, 10, 11, 12]) and dumped["periods"].dtype == np.float64
+    assert np.array_equal(dumped["background_clip0"], outputs[0][0])
+    assert np.array_equal(dumped["background_sample_positions"], positions)
+    assert np.array_equal(dumped["background_sample"], np.concatenate(outputs)[:, :, positions])
 
 
 def test_ragged_batches_are_grouped_by_shape_not_padded():
