@@ -67,8 +67,14 @@ int repet_set_stream(repet_handle* h, void* cuda_stream);
 /* Analysis window, HOST pointer, n = window length (built with SciPy's periodic Hamming by the
  * host, repet.py:131 -- SciPy's values differ from the closed form by up to 1 ulp). */
 int repet_set_window(repet_handle* h, const double* window, int n);
-/* Cap on the workspace (bytes) a batch call may use per chunk of clips; 0 = default. */
+/* Cap on the workspace (bytes) a batch call may use per chunk of clips; 0 = default (min(24 GiB, 40 % of the
+ * device memory free when the handle first asks)).  A chunk never holds less than one clip, so one clip whose
+ * workspace alone exceeds the cap still runs.  REPET-SIM honours the cap for long tracks too: when a track's
+ * similarity matrix does not fit, it is formed and consumed in row panels as high as the cap leaves room for
+ * (at least 128 rows), one track at a time.  Buffers an entry point stages its own input and output in come on top. */
 int repet_set_workspace_limit(repet_handle* h, uint64_t bytes);
+/* Bytes of device workspace the handle holds now (it grows on demand and is kept for later calls). */
+uint64_t repet_workspace_bytes(repet_handle* h);
 int repet_synchronize(repet_handle* h);
 /* Number of kernels this handle has launched since creation (bench.py's gpu_launches). */
 uint64_t repet_launch_count(repet_handle* h);

@@ -191,6 +191,8 @@ int repet_set_workspace_limit(repet_handle* h, uint64_t bytes) {
     return REPET_OK;
 }
 
+uint64_t repet_workspace_bytes(repet_handle* h) { return h ? (uint64_t)h->arena_bytes : 0; }
+
 int repet_synchronize(repet_handle* h) {
     if (!h) return REPET_E_INVALID_ARG;
     CU(cudaSetDevice(h->device));

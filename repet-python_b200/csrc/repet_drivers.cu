@@ -168,6 +168,8 @@ struct Plan {
     int seg_frames = 0, step_frames = 0, n_beat_seg = 0, left_pad = 0, lag_hi = 0, beat_parts = 0, beat_f_per_part = 0;
     // sim / simonline
     int number = 0, distance = 0, buffer_frames = 0;
+    // sim: height of the row panels S is formed in (a multiple of 128), 0 = the whole matrix at once
+    int panel_rows = 0;
     int ints_per_clip = 1;
     size_t bytes_per_clip = 0;
 };
@@ -272,9 +274,24 @@ int make_plan(repet_handle* h, int kind, const repet_params* p, int nch, int64_t
         if (plan->number > 32) b += align_up((size_t)nch * T * PPITCH * sizeof(float));  // squared magnitudes
         if (kind == KIND_SIM) {
             b += 2 * align_up((size_t)T * KPAD * sizeof(float));  // An32 hi, lo
-            b += align_up((size_t)T * T * sizeof(float));     // S
             b += align_up((size_t)T * sizeof(int32_t));       // columns handed to the exact fallback
             b += align_up(topk_exact_scratch_bytes(T, h->sm_count));
+            b += 2048;
+            // S: the whole matrix when it fits the workspace limit with the linear part above; otherwise row panels
+            // of as many rows as the limit leaves room for (128 when the linear part alone exceeds it), one track
+            // per chunk
+            const size_t row_bytes = (size_t)T * sizeof(float);
+            const size_t whole = align_up((size_t)T * row_bytes);
+            const size_t limit = default_ws_limit(h);
+            plan->panel_rows = 0;
+            if (b + whole > limit) {
+                const size_t room = limit > b + 256 ? (limit - b - 256) / row_bytes : 0;
+                const int P = (int)std::max<size_t>(128, std::min<size_t>(room, (size_t)T) / 128 * 128);
+                if (P < T) plan->panel_rows = P;
+            }
+            b += plan->panel_rows ? align_up((size_t)plan->panel_rows * row_bytes) : whole;
+            plan->bytes_per_clip = b;
+            return REPET_OK;
         }
         b += 2048;
         plan->bytes_per_clip = b;
@@ -298,8 +315,9 @@ int run_sim(repet_handle* h, const Plan& plan, const float* audio, int n_clips, 
             unsigned char* ws, size_t ws_bytes) {
     const int nch = plan.nch, T = plan.T;
     const bool online = plan.kind == KIND_SIMONLINE;
-    const int G = (int)std::min<size_t>(std::min<size_t>((size_t)n_clips, MAX_ITEMS_PER_LAUNCH / 2),
-                                        std::max<size_t>(1, ws_bytes / plan.bytes_per_clip));
+    const int P = online ? 0 : plan.panel_rows;  // row panels: one track per chunk
+    const int G = P ? 1 : (int)std::min<size_t>(std::min<size_t>((size_t)n_clips, MAX_ITEMS_PER_LAUNCH / 2),
+                                                std::max<size_t>(1, ws_bytes / plan.bytes_per_clip));
     const float scale = (float)(1.0 / ((double)WIN_N * plan.p.cola_gain));
     cudaStream_t st = h->stream;
     for (int clip0 = 0; clip0 < n_clips; clip0 += G) {
@@ -316,7 +334,7 @@ int run_sim(repet_handle* h, const Plan& plan, const float* audio, int n_clips, 
         float* An32 = online ? nullptr : bump.take<float>((size_t)g * T * KPAD);
         float* An32lo = online ? nullptr : bump.take<float>((size_t)g * T * KPAD);
         const int fast = g_tuning.simgemm_tc;
-        float* S = online ? nullptr : bump.take<float>((size_t)g * T * T);
+        float* S = online ? nullptr : bump.take<float>(P ? (size_t)P * T : (size_t)g * T * T);
         int32_t* ovf_cols = online ? nullptr : bump.take<int32_t>((size_t)g * T);
         unsigned char* ovf_scratch = online ? nullptr : bump.take<unsigned char>(topk_exact_scratch_bytes(T, h->sm_count));
         Geom geom = clip_geom(g, nch, plan.S, T);
@@ -349,20 +367,49 @@ int run_sim(repet_handle* h, const Plan& plan, const float* audio, int n_clips, 
                                      plan.p.similarity_threshold, plan.distance, plan.number, idx, cnt))
                 return fail(h, REPET_E_UNSUPPORTED, "buffer_length too long for the online selection kernel on this device");
         } else {
-            {
-                Timed timed(h, REPET_K_SIMGEMM);
-                if (fast) {
-                    if (launch_selfsim_tc(st, An32, fast >= 2 ? An32lo : nullptr, g, T, S, h->sm_count))
-                        return fail(h, REPET_E_CUDA, "tensor-map encode failed for the similarity GEMM");
-                } else {
-                    launch_selfsim_simt(st, An32, g, T, S);
+            const float tau = fast >= 2 ? TAU_3XTF32_GEMM : (fast ? TAU_TF32_GEMM : TAU_FP32_GEMM);
+            const double thr = plan.p.similarity_threshold;
+            if (!P) {
+                {
+                    Timed timed(h, REPET_K_SIMGEMM);
+                    if (fast) {
+                        if (launch_selfsim_tc(st, An32, fast >= 2 ? An32lo : nullptr, g, T, S, h->sm_count))
+                            return fail(h, REPET_E_CUDA, "tensor-map encode failed for the similarity GEMM");
+                    } else {
+                        launch_selfsim_simt(st, An32, g, T, S);
+                    }
                 }
+                CU(cudaMemsetAsync(overflow, 0, 4 * sizeof(int32_t), st));
+                Timed timed(h, REPET_K_TOPK, 2);  // k_topk, k_topk_exact
+                if (launch_topk_propose(st, S, 0, T, An64, g, T, tau, thr, plan.distance, plan.number, idx, cnt, overflow,
+                                        ovf_cols))
+                    return fail(h, REPET_E_UNSUPPORTED, "similarity_distance too large for the in-shared-memory similarity row");
+                launch_topk_exact(st, An64, T, thr, plan.distance, plan.number, overflow, ovf_cols, ovf_scratch, idx, cnt,
+                                  h->sm_count);
+            } else {
+                // rows [r0, r0 + P) of S, then the columns they settle; the columns k_topk queues for the exact
+                // fallback accumulate over the panels and are settled once at the end
+                CU(cudaMemsetAsync(overflow, 0, 4 * sizeof(int32_t), st));
+                for (int r0 = 0; r0 < T; r0 += P) {
+                    const int rows = std::min(P, T - r0);
+                    {
+                        Timed timed(h, REPET_K_SIMGEMM);
+                        if (fast) {
+                            if (launch_selfsim_tc_panel(st, An32, fast >= 2 ? An32lo : nullptr, T, r0, rows, S, h->sm_count))
+                                return fail(h, REPET_E_CUDA, "tensor-map encode failed for the similarity GEMM");
+                        } else {
+                            launch_selfsim_simt_panel(st, An32, T, r0, rows, S);
+                        }
+                    }
+                    Timed timed(h, REPET_K_TOPK);
+                    if (launch_topk_propose(st, S, r0, rows, An64, 1, T, tau, thr, plan.distance, plan.number, idx, cnt,
+                                            overflow, ovf_cols))
+                        return fail(h, REPET_E_UNSUPPORTED, "similarity_distance too large for the in-shared-memory similarity row");
+                }
+                Timed timed(h, REPET_K_TOPK);
+                launch_topk_exact(st, An64, T, thr, plan.distance, plan.number, overflow, ovf_cols, ovf_scratch, idx, cnt,
+                                  h->sm_count);
             }
-            CU(cudaMemsetAsync(overflow, 0, 4 * sizeof(int32_t), st));
-            Timed timed(h, REPET_K_TOPK, 2);  // k_topk, k_topk_exact
-            if (launch_topk(st, S, An64, g, T, fast >= 2 ? TAU_3XTF32_GEMM : (fast ? TAU_TF32_GEMM : TAU_FP32_GEMM), plan.p.similarity_threshold, plan.distance, plan.number,
-                            idx, cnt, overflow, ovf_cols, ovf_scratch, h->sm_count))
-                return fail(h, REPET_E_UNSUPPORTED, "track too long for the in-shared-memory similarity row");
         }
         {
             Timed timed(h, REPET_K_MODEL, Vsq ? 3 : 2);  // k_simmodel, [k_simmodel_large,] k_simmodel_nyquist
@@ -380,7 +427,8 @@ int run_sim(repet_handle* h, const Plan& plan, const float* audio, int n_clips, 
             CU(cudaMemcpyAsync(flag, overflow, sizeof(flag), cudaMemcpyDeviceToHost, st));
             CU(cudaStreamSynchronize(st));
             fprintf(stderr, "k_topk: %d columns (%d through the exact fallback), %d candidates, %d uncertain, %d near-tie "
-                            "neighbour dots\n", g * T, flag[0], flag[1], flag[2], flag[3]);
+                            "neighbour dots; %d row panels of %d\n", g * T, flag[0], flag[1], flag[2], flag[3],
+                    P ? (T + P - 1) / P : 1, P ? P : T);
         }
     }
     CU(cudaGetLastError());
@@ -502,6 +550,7 @@ int run_plan(repet_handle* h, const Plan& plan, const float* audio, int n_clips,
 }
 
 int chunk_clips(repet_handle* h, const Plan& plan, int n_clips) {
+    if (plan.panel_rows) return std::min(n_clips, 1);  // a track in row panels runs alone
     const size_t limit = default_ws_limit(h);
     return (int)std::min<size_t>((size_t)n_clips, std::max<size_t>(1, limit / plan.bytes_per_clip));
 }

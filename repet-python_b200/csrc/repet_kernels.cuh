@@ -164,11 +164,20 @@ void launch_frames64(cudaStream_t st, const float* audio, const double* audio64,
 // tcgen05 / TMEM / TMA self-similarity GEMM (repet_simgemm.cu); returns 0 on success
 int launch_selfsim_tc(cudaStream_t st, const float* hi, const float* lo, int n_items, int T, float* S, int sm_count);
 void launch_selfsim_simt(cudaStream_t st, const float* An32, int n_items, int T, float* S);
-// overflow: [4] ints zeroed by the caller ([0] = columns handed to the exact fallback, [1..3] statistics);
-// ovf_cols: [n_items * T] ints; scratch: topk_exact_scratch_bytes(T, sm_count) bytes
-int launch_topk(cudaStream_t st, const float* S, const double* An64, int n_items, int T, float tau, double thr, int d,
-                int number, int* idx_out, int* cnt_out, int* overflow, int* ovf_cols, unsigned char* scratch,
-                int sm_count);
+// rows [r0, r0 + rows) of one item's S, row-major with pitch T (S_panel[r - r0][c])
+int launch_selfsim_tc_panel(cudaStream_t st, const float* hi, const float* lo, int T, int r0, int rows, float* S_panel,
+                            int sm_count);
+void launch_selfsim_simt_panel(cudaStream_t st, const float* An32, int T, int r0, int rows, float* S_panel);
+// The similar-frame selection in two launches.  k_topk settles columns [c0, c0 + n_cols) of every item from the rows
+// S[(item * n_cols + c - c0) * T ...] (the whole matrix: c0 = 0, n_cols = T; a row panel of one item: its first row
+// and height) and queues the columns it cannot settle; k_topk_exact then settles every queued column, once after the
+// last panel.  overflow: [4] ints zeroed by the caller ([0] = columns queued for the exact fallback, [1..3]
+// statistics); ovf_cols: [n_items * T] ints; scratch: topk_exact_scratch_bytes(T, sm_count) bytes.
+int launch_topk_propose(cudaStream_t st, const float* S, int c0, int n_cols, const double* An64, int n_items, int T,
+                        float tau, double thr, int d, int number, int* idx_out, int* cnt_out, int* overflow,
+                        int* ovf_cols);
+void launch_topk_exact(cudaStream_t st, const double* An64, int T, double thr, int d, int number, const int* overflow,
+                       const int* ovf_cols, unsigned char* scratch, int* idx_out, int* cnt_out, int sm_count);
 size_t topk_exact_scratch_bytes(int T, int sm_count);
 // returns 0, or nonzero when the device refuses the shared memory / scratch the ring needs
 int launch_online_select(cudaStream_t st, const double* An64, int n_items, int T, int B, int frame_base, double thr,

@@ -227,15 +227,17 @@ void launch_frames64(cudaStream_t st, const float* audio, const double* audio64,
 // 64x64 output tile per CTA, 16x16 threads x 4x4 accumulators, K in chunks of 16 through smem.
 // The products are summed in the same k order for (i, j) and (j, i): S is bitwise symmetric.
 // ------------------------------------------------------------------------------------------
+// Output rows j in [r0, r0 + rows) (the whole matrix: r0 = 0, rows = T) at Sout[(j - r0) * T + i].
 __global__ void __launch_bounds__(256)
-k_selfsim_simt(const float* __restrict__ An32, int T, float* __restrict__ S) {
+k_selfsim_simt(const float* __restrict__ An32, int T, int r0, int rows, float* __restrict__ S) {
     __shared__ float sa[16][65];
     __shared__ float sb[16][65];
     const int item = blockIdx.z;
     const float* __restrict__ A = An32 + (size_t)item * T * KPAD;
-    float* __restrict__ Sout = S + (size_t)item * T * T;
+    float* __restrict__ Sout = S + (size_t)item * rows * T;
     const int ti = threadIdx.x & 15, tj = threadIdx.x >> 4;
-    const int i0 = blockIdx.y * 64, j0 = blockIdx.x * 64;
+    const int i0 = blockIdx.y * 64, j0 = r0 + blockIdx.x * 64;
+    const int j_end = r0 + rows;
     float acc[4][4];
 #pragma unroll
     for (int a = 0; a < 4; ++a)
@@ -249,7 +251,7 @@ k_selfsim_simt(const float* __restrict__ An32, int T, float* __restrict__ S) {
             const int row = idx >> 4, kk = idx & 15;
             const int ri = i0 + row, rj = j0 + row;
             sa[kk][row] = ri < T ? A[(size_t)ri * KPAD + k0 + kk] : 0.f;
-            sb[kk][row] = rj < T ? A[(size_t)rj * KPAD + k0 + kk] : 0.f;
+            sb[kk][row] = rj < j_end ? A[(size_t)rj * KPAD + k0 + kk] : 0.f;
         }
         __syncthreads();
 #pragma unroll
@@ -271,13 +273,19 @@ k_selfsim_simt(const float* __restrict__ An32, int T, float* __restrict__ S) {
 #pragma unroll
         for (int b = 0; b < 4; ++b) {
             const int i = i0 + ti + 16 * a, j = j0 + tj + 16 * b;
-            if (i < T && j < T) Sout[(size_t)j * T + i] = acc[a][b];
+            if (i < T && j < j_end) Sout[(size_t)(j - r0) * T + i] = acc[a][b];
         }
 }
 
 void launch_selfsim_simt(cudaStream_t st, const float* An32, int n_items, int T, float* S) {
     dim3 grid((T + 63) / 64, (T + 63) / 64, n_items);
-    k_selfsim_simt<<<grid, 256, 0, st>>>(An32, T, S);
+    k_selfsim_simt<<<grid, 256, 0, st>>>(An32, T, 0, T, S);
+}
+
+// the same products as the whole matrix, so a panel holds exactly the whole matrix's rows
+void launch_selfsim_simt_panel(cudaStream_t st, const float* An32, int T, int r0, int rows, float* S_panel) {
+    dim3 grid((rows + 63) / 64, (T + 63) / 64, 1);
+    k_selfsim_simt<<<grid, 256, 0, st>>>(An32, T, r0, rows, S_panel);
 }
 
 constexpr int DOTN = (NBIN + 31) / 32;  // elements of a frame per lane
@@ -332,13 +340,136 @@ constexpr int TOPK_THREADS = REPET_TOPK_THREADS;
 constexpr int TOPK_CAP = REPET_TOPK_CAP;       // candidates per column held in shared memory
 constexpr int TOPK_CHUNK = REPET_TOPK_CHUNK;   // elements of the fast row resident at a time (3 arrays)
 constexpr int TOPK_BINS = 512;       // histogram of fast values over [-1, 1) for the top-`number` cut
+// candidates held before the running prune cuts the buffer (checked at chunk boundaries: one chunk of a row proposes
+// at most about payload / (d + 1) certain candidates, far below the remaining TOPK_CAP - TOPK_FILL for d of a second)
+constexpr int TOPK_FILL = TOPK_CAP * 3 / 4;
 __device__ __forceinline__ int topk_bin(float v) {
     return min(TOPK_BINS - 1, max(0, (int)floorf((v + 1.f) * (TOPK_BINS / 2.f))));
 }
 
+// ---- prune: only the `number` best survive the ranking -------------------------------------------
+// Let c be a value that at least `number` CERTAIN candidates (kept whatever the exact values say) reach in the fast
+// pass.  A candidate with v~ < c - 2 tau is exactly below all of them, so it can never be written; it needs no exact
+// value and takes no part in the ranking.  c comes from a histogram of the certain candidates (bin width 2^-8),
+// conservative by up to one bin.  REFINE (the running prune of long rows, whose maxima crowd the bins near the cut)
+// splits that bin into TOPK_BINS sub-bins of 2^-17 with a second histogram, so c is conservative by 2^-17 instead.
+// Compacts s_cand / s_vc to the candidates at or above the cut and returns their count; *s_cut is the cut (-inf:
+// fewer than `number` certain candidates, nothing pruned).  Every thread of the CTA calls it with the same count;
+// s_hist is TOPK_BINS ints of free shared memory, s_sel two ints.
+template <bool REFINE>
+__device__ int topk_prune(int count, int number, float two_tau, int* s_cand, float* s_vc, int* s_hist, float* s_cut,
+                          int* s_count, int* s_sel) {
+    const int t = threadIdx.x, lane = t & 31, warp = t >> 5;
+    for (int b = t; b < TOPK_BINS; b += blockDim.x) s_hist[b] = 0;
+    __syncthreads();
+    for (int q = t; q < count; q += blockDim.x)
+        if (!(s_cand[q] & (1 << 30))) atomicAdd(&s_hist[topk_bin(s_vc[q])], 1);
+    __syncthreads();
+    if (warp == 0) {
+        constexpr int PER_LANE = TOPK_BINS / 32;
+        int mine = 0;
+#pragma unroll
+        for (int u = 0; u < PER_LANE; ++u) mine += s_hist[lane * PER_LANE + u];
+        int above = 0;  // certain candidates in the bins of higher lanes
+#pragma unroll
+        for (int o = 0; o < 32; ++o) {
+            const int other = __shfl_sync(0xffffffffu, mine, o);
+            if (o > lane) above += other;
+        }
+        const bool holds = above < number && above + mine >= number;
+        const unsigned who = __ballot_sync(0xffffffffu, holds);
+        if (who == 0) {
+            if (lane == 0) {
+                *s_cut = -INFINITY;  // fewer than `number` certain candidates: nothing to prune
+                if (REFINE) s_sel[0] = -1;
+            }
+        } else if (lane == __ffs(who) - 1) {
+            int cum = above, b = lane * PER_LANE + PER_LANE - 1;
+            for (; b > lane * PER_LANE; --b) {
+                cum += s_hist[b];
+                if (cum >= number) break;
+            }
+            if (REFINE && b == lane * PER_LANE && cum < number) cum += s_hist[b];  // the loop stops before the lane's last bin
+            *s_cut = (float)b * (2.f / TOPK_BINS) - 1.f - two_tau - 1e-6f;  // lower edge of the bin, minus 2 tau (and binning rounding)
+            if (REFINE) {
+                s_sel[0] = b;
+                s_sel[1] = cum - s_hist[b];  // certain candidates above bin b
+            }
+        }
+    }
+    __syncthreads();
+    if (REFINE && s_sel[0] >= 0) {  // the same value in every thread
+        const int b = s_sel[0], base = s_sel[1];
+        const float lo = (float)b * (2.f / TOPK_BINS) - 1.f;
+        constexpr float SUB_SCALE = (float)TOPK_BINS * TOPK_BINS / 2.f;  // sub-bins per unit of v
+        __syncthreads();  // every thread has read s_sel before the histogram is reused
+        for (int u = t; u < TOPK_BINS; u += blockDim.x) s_hist[u] = 0;
+        __syncthreads();
+        for (int q = t; q < count; q += blockDim.x) {
+            const float v = s_vc[q];
+            if (!(s_cand[q] & (1 << 30)) && topk_bin(v) == b)
+                atomicAdd(&s_hist[min(TOPK_BINS - 1, max(0, (int)floorf((v - lo) * SUB_SCALE)))], 1);
+        }
+        __syncthreads();
+        if (warp == 0) {
+            constexpr int PER_LANE = TOPK_BINS / 32;
+            int mine = 0;
+#pragma unroll
+            for (int u = 0; u < PER_LANE; ++u) mine += s_hist[lane * PER_LANE + u];
+            int above = base;
+#pragma unroll
+            for (int o = 0; o < 32; ++o) {
+                const int other = __shfl_sync(0xffffffffu, mine, o);
+                if (o > lane) above += other;
+            }
+            const bool holds = above < number && above + mine >= number;
+            const unsigned who = __ballot_sync(0xffffffffu, holds);
+            if (who != 0 && lane == __ffs(who) - 1) {  // none: keep the bin's own cut
+                int cum = above, sb = lane * PER_LANE + PER_LANE - 1;
+                for (; sb > lane * PER_LANE; --sb) {
+                    cum += s_hist[sb];
+                    if (cum >= number) break;
+                }
+                *s_cut = lo + (float)sb / SUB_SCALE - two_tau - 1e-6f;  // lower edge of the sub-bin, minus 2 tau
+            }
+        }
+        __syncthreads();
+    }
+    const float cut = *s_cut;
+    if (cut > -INFINITY) {
+        // compact the survivors in place (one warp, chunks of 32 in order: writes never pass reads)
+        if (warp == 0) {
+            int kept = 0;
+            for (int q0 = 0; q0 < count; q0 += 32) {
+                const int q = q0 + lane;
+                const int code = q < count ? s_cand[q] : 0;
+                const float v = q < count ? s_vc[q] : 0.f;
+                const bool keep = q < count && v >= cut;
+                const unsigned m = __ballot_sync(0xffffffffu, keep);
+                __syncwarp();
+                if (keep) {
+                    const int pos = kept + __popc(m & ((1u << lane) - 1));
+                    s_cand[pos] = code;
+                    s_vc[pos] = v;
+                }
+                kept += __popc(m);
+                __syncwarp();
+            }
+            if (lane == 0) *s_count = kept;
+        }
+        __syncthreads();
+        count = *s_count;
+    }
+    return count;
+}
+
+// Column c = c0 + blockIdx.x reads its fast row at S + (item * gridDim.x + blockIdx.x) * T: the whole matrix
+// (c0 = 0, gridDim.x = T) or a row panel of one item (c0 = its first row).  Outputs are indexed by the absolute column.
+// RUNNING: the running prune below, compiled in for rows that can hold more than TOPK_CAP maxima.
+template <bool RUNNING>
 __global__ void __launch_bounds__(TOPK_THREADS)
-k_topk(const float* __restrict__ S, const double* __restrict__ An64, int T, float tau, double thr, int d, int number,
-       int nb, int* __restrict__ idx_out, int* __restrict__ cnt_out, int* __restrict__ overflow,
+k_topk(const float* __restrict__ S, int c0, const double* __restrict__ An64, int T, float tau, double thr, int d,
+       int number, int nb, int* __restrict__ idx_out, int* __restrict__ cnt_out, int* __restrict__ overflow,
        int* __restrict__ ovf_cols, int force_exact) {
     extern __shared__ __align__(16) unsigned char smem[];
     double* s_col = reinterpret_cast<double*>(smem);           // [APITCH64]   column c, float64
@@ -348,11 +479,11 @@ k_topk(const float* __restrict__ S, const double* __restrict__ An64, int T, floa
     float* s_e = s_vc + TOPK_CAP;                              // [nb*d]       extended chunk of the fast row
     float* s_pm = s_e + TOPK_CHUNK;                            // prefix maxima within blocks of d
     float* s_sm = s_pm + TOPK_CHUNK;                           // suffix maxima within blocks of d
-    __shared__ int s_count, s_kept;
+    __shared__ int s_count, s_kept, s_sel[2];
     __shared__ float s_cut;
-    const int item = blockIdx.y, c = blockIdx.x;
+    const int item = blockIdx.y, c = c0 + blockIdx.x;
     const int t = threadIdx.x, lane = t & 31, warp = t >> 5, nwarp = blockDim.x >> 5;
-    const float* __restrict__ row = S + ((size_t)item * T + c) * (size_t)T;
+    const float* __restrict__ row = S + ((size_t)item * gridDim.x + blockIdx.x) * (size_t)T;
     const double* __restrict__ A = An64 + (size_t)item * T * APITCH64;
     if (force_exact) {  // test knob: every column goes through k_topk_exact
         if (t == 0) ovf_cols[atomicAdd(overflow, 1)] = item * T + c;
@@ -381,9 +512,23 @@ k_topk(const float* __restrict__ S, const double* __restrict__ An64, int T, floa
             nxt[u] = (x < ext && g >= 0 && g < T) ? __ldg(row + g) : -INFINITY;
         }
     };
+    // Running prune: a long row proposes more local maxima than the buffer holds (about one per 2 d frames).  When
+    // the buffer passes TOPK_FILL at a chunk boundary, topk_prune cuts it down to what can still be among the
+    // `number` best, and later proposals below that cut are dropped.  The cut only rises as certain candidates
+    // arrive, so a dropped proposal stays exactly below `number` certain ones.  It is compiled in only for rows that
+    // can hold more than TOPK_CAP maxima d + 1 frames apart (launch_topk_propose); shorter rows can overflow only
+    // through near-ties, which is what k_topk_exact is for, and run exactly the kernel they ran before.
+    float run_cut = -INFINITY;
     fetch(0);
     for (int g0 = 0; g0 < T; g0 += payload) {
         __syncthreads();
+        if (RUNNING && g0 > 0) {  // every proposal of the previous chunk is in; s_pm / s_sm are free until the staging
+            const int n = s_count;
+            if (n > TOPK_FILL && n <= TOPK_CAP && n > number) {
+                topk_prune<true>(n, number, two_tau, s_cand, s_vc, reinterpret_cast<int*>(s_pm), &s_cut, &s_count, s_sel);
+                run_cut = fmaxf(run_cut, s_cut);
+            }
+        }
 #pragma unroll
         for (int u = 0; u < PER_THREAD; ++u) {
             const int x = t + u * TOPK_THREADS;
@@ -414,6 +559,7 @@ k_topk(const float* __restrict__ S, const double* __restrict__ An64, int T, floa
             const int xe = d > 0 ? x + d : x;
             const float v = s_e[xe];
             if (!(v >= thr_f - tau) || !(v < INFINITY)) continue;
+            if (RUNNING && v < run_cut) continue;  // below `number` certain candidates already held
             float m = -INFINITY;
             if (d > 0) {
                 // left window [xe-d, xe-1] and right window [xe+1, xe+d]: each exactly one block long
@@ -439,69 +585,9 @@ k_topk(const float* __restrict__ S, const double* __restrict__ An64, int T, floa
         return;
     }
     if (t == 0) atomicAdd(overflow + 1, count);  // statistics: candidates proposed
-    // ---- prune: only the `number` best survive the ranking ---------------------------------------
-    // Let c be a value that at least `number` CERTAIN candidates (kept whatever the exact values say)
-    // reach in the fast pass.  A candidate with v~ < c - 2 tau is exactly below all of them, so it can
-    // never be written; it needs no exact value and takes no part in the ranking.  c comes from a
-    // histogram of the certain candidates (bin width 2^-8), conservative by up to one bin.
-    if (count > number) {
-        int* s_hist = reinterpret_cast<int*>(s_pm);  // the chunk buffers are free now
-        for (int b = t; b < TOPK_BINS; b += blockDim.x) s_hist[b] = 0;
-        __syncthreads();
-        for (int q = t; q < count; q += blockDim.x)
-            if (!(s_cand[q] & (1 << 30))) atomicAdd(&s_hist[topk_bin(s_vc[q])], 1);
-        __syncthreads();
-        if (warp == 0) {
-            constexpr int PER_LANE = TOPK_BINS / 32;
-            int mine = 0;
-#pragma unroll
-            for (int u = 0; u < PER_LANE; ++u) mine += s_hist[lane * PER_LANE + u];
-            int above = 0;  // certain candidates in the bins of higher lanes
-#pragma unroll
-            for (int o = 0; o < 32; ++o) {
-                const int other = __shfl_sync(0xffffffffu, mine, o);
-                if (o > lane) above += other;
-            }
-            const bool holds = above < number && above + mine >= number;
-            const unsigned who = __ballot_sync(0xffffffffu, holds);
-            if (who == 0) {
-                if (lane == 0) s_cut = -INFINITY;  // fewer than `number` certain candidates: nothing to prune
-            } else if (lane == __ffs(who) - 1) {
-                int cum = above, b = lane * PER_LANE + PER_LANE - 1;
-                for (; b > lane * PER_LANE; --b) {
-                    cum += s_hist[b];
-                    if (cum >= number) break;
-                }
-                s_cut = (float)b * (2.f / TOPK_BINS) - 1.f - two_tau - 1e-6f;  // lower edge of the bin, minus 2 tau (and binning rounding)
-            }
-        }
-        __syncthreads();
-        const float cut = s_cut;
-        if (cut > -INFINITY) {
-            // compact the survivors in place (one warp, chunks of 32 in order: writes never pass reads)
-            if (warp == 0) {
-                int kept = 0;
-                for (int q0 = 0; q0 < count; q0 += 32) {
-                    const int q = q0 + lane;
-                    const int code = q < count ? s_cand[q] : 0;
-                    const float v = q < count ? s_vc[q] : 0.f;
-                    const bool keep = q < count && v >= cut;
-                    const unsigned m = __ballot_sync(0xffffffffu, keep);
-                    __syncwarp();
-                    if (keep) {
-                        const int pos = kept + __popc(m & ((1u << lane) - 1));
-                        s_cand[pos] = code;
-                        s_vc[pos] = v;
-                    }
-                    kept += __popc(m);
-                    __syncwarp();
-                }
-                if (lane == 0) s_count = kept;
-            }
-            __syncthreads();
-            count = s_count;
-        }
-    }
+    // ---- prune: only the `number` best survive the ranking (topk_prune) -------------------------
+    if (count > number)
+        count = topk_prune<false>(count, number, two_tau, s_cand, s_vc, reinterpret_cast<int*>(s_pm), &s_cut, &s_count, s_sel);
     // ---- which candidates need their exact value? ---------------------------------------------
     // the uncertain ones (local-maximum test within 2 tau) and every pair whose fast values are within
     // 2 tau of each other (their ORDER is not decided by the fast pass); bit 29 marks them
@@ -637,11 +723,9 @@ size_t topk_exact_scratch_bytes(int T, int sm_count) {
     return per_cta * (size_t)(sm_count * TOPK_EXACT_CTAS_PER_SM);
 }
 
-// ovf_cols: [n_items * T] ints; scratch: topk_exact_scratch_bytes(T, sm_count) bytes; overflow[0] counts the
-// columns handed to the exact kernel (zeroed by the caller)
-int launch_topk(cudaStream_t st, const float* S, const double* An64, int n_items, int T, float tau, double thr, int d,
-                int number, int* idx_out, int* cnt_out, int* overflow, int* ovf_cols, unsigned char* scratch,
-                int sm_count) {
+int launch_topk_propose(cudaStream_t st, const float* S, int c0, int n_cols, const double* An64, int n_items, int T,
+                        float tau, double thr, int d, int number, int* idx_out, int* cnt_out, int* overflow,
+                        int* ovf_cols) {
     // blocks of d elements per chunk: as many as fit, at least halo + one payload block
     int nb = 3;
     if (d > 0) {
@@ -649,15 +733,28 @@ int launch_topk(cudaStream_t st, const float* S, const double* An64, int n_items
         if (nb < 3) return -1;  // similarity_distance too large for the shared-memory window
     }
     const size_t smem = (size_t)APITCH64 * 8 + (size_t)TOPK_CAP * 16 + 3 * (size_t)TOPK_CHUNK * 4;
-    static SmemOptIn opt_in;
-    smem_opt_in(k_topk, smem, opt_in);
-    dim3 grid(T, n_items);
-    k_topk<<<grid, TOPK_THREADS, smem, st>>>(S, An64, T, tau, thr, d, number, nb, idx_out, cnt_out, overflow, ovf_cols,
-                                             g_tuning.topk_force_exact);
+    dim3 grid(n_cols, n_items);
+    // the running prune pays for rows that can hold more than TOPK_CAP maxima (strict maxima within +-d are more
+    // than d frames apart): at similarity_distance 1 s, tracks above about 13 minutes
+    if ((long long)T > (long long)(d + 1) * TOPK_CAP) {
+        static SmemOptIn opt_in;
+        smem_opt_in(k_topk<true>, smem, opt_in);
+        k_topk<true><<<grid, TOPK_THREADS, smem, st>>>(S, c0, An64, T, tau, thr, d, number, nb, idx_out, cnt_out,
+                                                       overflow, ovf_cols, g_tuning.topk_force_exact);
+    } else {
+        static SmemOptIn opt_in;
+        smem_opt_in(k_topk<false>, smem, opt_in);
+        k_topk<false><<<grid, TOPK_THREADS, smem, st>>>(S, c0, An64, T, tau, thr, d, number, nb, idx_out, cnt_out,
+                                                        overflow, ovf_cols, g_tuning.topk_force_exact);
+    }
+    return 0;
+}
+
+void launch_topk_exact(cudaStream_t st, const double* An64, int T, double thr, int d, int number, const int* overflow,
+                       const int* ovf_cols, unsigned char* scratch, int* idx_out, int* cnt_out, int sm_count) {
     const size_t per_cta = ((size_t)T * 12 + 255) / 256 * 256;
     k_topk_exact<<<sm_count * TOPK_EXACT_CTAS_PER_SM, TOPK_THREADS, 0, st>>>(An64, T, thr, d, number, overflow, ovf_cols,
                                                                             scratch, per_cta, idx_out, cnt_out);
-    return 0;
 }
 
 // ------------------------------------------------------------------------------------------

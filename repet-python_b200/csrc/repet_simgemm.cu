@@ -13,7 +13,8 @@
 //               smem tile so that global stores are 128-byte coalesced rows, predicated on the
 //               ragged edges; overlaps the next tile's MMAs through the second accumulator
 // In the split configuration only the tiles that reach the diagonal or lie above it are computed; the epilogue
-// writes every element above the diagonal and its mirror image.
+// writes every element above the diagonal and its mirror image.  A row panel (tracks whose S exceeds the workspace
+// limit) is computed as a full rectangle in both configurations.
 // The result only PROPOSES similar-frame candidates: k_topk certifies every decision with exact
 // float64 dot products, with tau covering the TF32 rounding (|S~ - S| <= 2 * 2^-11 + accumulation).
 #include "repet_kernels.cuh"
@@ -155,13 +156,22 @@ __host__ __device__ inline int triangle_tiles(int mt, int nt) {
     return total;
 }
 
+// Without the triangle: row-major over the whole matrix, or (a row panel, `col_raster`) column by column -- all tile
+// rows of a tile column before the next, so the panel's own operand rows stay in L2 while every other operand block
+// is read once per panel (the band argument above with the panel as the band).
 template <bool TRI, int Q>
-__device__ __forceinline__ void decode_tile(int tile, int per_item, int mt, int nt, int& item, int& mi, int& ni) {
+__device__ __forceinline__ void decode_tile(int tile, int per_item, int mt, int nt, bool col_raster, int& item, int& mi,
+                                            int& ni) {
     if (!TRI) {
         item = tile / (mt * nt);
         const int rem = tile - item * (mt * nt);
-        mi = rem / nt;
-        ni = rem - mi * nt;
+        if (col_raster) {
+            ni = rem / mt;
+            mi = rem - ni * mt;
+        } else {
+            mi = rem / nt;
+            ni = rem - mi * nt;
+        }
         return;
     }
     item = tile / per_item;
@@ -187,11 +197,13 @@ __device__ __forceinline__ void decode_tile(int tile, int per_item, int mt, int 
     ni = (RASTER_G / Q) * band + c;
 }
 
-template <int BN, bool SPLIT3>
+// Rows [r0, r0 + rows) of S for every item: element (row, col) at S[(item * rows + row - r0) * T + col].  The whole
+// matrix is r0 = 0, rows = T; TRI (the triangle with mirror writes) needs the whole matrix.
+template <int BN, bool SPLIT3, bool TRI>
 __global__ void __launch_bounds__(GEMM_THREADS, 1)
 k_simgemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b,
-          const __grid_constant__ CUtensorMap map_a_lo, const __grid_constant__ CUtensorMap map_b_lo, int T, int n_items,
-          int per_item, float* __restrict__ S) {
+          const __grid_constant__ CUtensorMap map_a_lo, const __grid_constant__ CUtensorMap map_b_lo, int T, int r0,
+          int rows, int n_items, int per_item, int col_raster, float* __restrict__ S) {
     using Cfg = GemmCfg<BN, SPLIT3>;
     constexpr int STAGES = Cfg::STAGES;
     constexpr int B_BYTES = Cfg::B_BYTES;
@@ -209,9 +221,9 @@ k_simgemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
     uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(acc_empty + 2);
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    constexpr bool TRI = SPLIT3;  // the split configuration forms the triangle only
     constexpr int Q = BN / BM;
-    const int mt = (T + BM - 1) / BM, nt = (T + BN - 1) / BN;
+    const int mt = (rows + BM - 1) / BM, nt = (T + BN - 1) / BN;
+    const int row_end = r0 + rows;
     const int tiles_total = n_items * per_item;
 
     if (threadIdx.x == 0) {
@@ -242,8 +254,8 @@ k_simgemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
             uint32_t it = 0;
             for (int tile = blockIdx.x; tile < tiles_total; tile += gridDim.x) {
                 int item, mi, ni;
-                decode_tile<TRI, Q>(tile, per_item, mt, nt, item, mi, ni);
-                const int m0 = mi * BM, n0 = ni * BN;
+                decode_tile<TRI, Q>(tile, per_item, mt, nt, col_raster, item, mi, ni);
+                const int m0 = r0 + mi * BM, n0 = ni * BN;
                 for (int kb = 0; kb < KBLOCKS; ++kb, ++it) {
                     const int s = it % STAGES;
                     mbar_wait(&empty[s], ((it / STAGES) & 1) ^ 1);
@@ -297,8 +309,8 @@ k_simgemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
         uint32_t tile_iter = 0;
         for (int tile = blockIdx.x; tile < tiles_total; tile += gridDim.x, ++tile_iter) {
             int item, mi, ni;
-            decode_tile<TRI, Q>(tile, per_item, mt, nt, item, mi, ni);
-            const int m0 = mi * BM, n0 = ni * BN;
+            decode_tile<TRI, Q>(tile, per_item, mt, nt, col_raster, item, mi, ni);
+            const int m0 = r0 + mi * BM, n0 = ni * BN;
             // every element of S is written exactly once: (row, col) with col >= row directly, its mirror image
             // from the same registers; the part of a diagonal-crossing tile below the diagonal is dropped
             const bool crosses = TRI && n0 < m0 + BM;  // the tile holds elements on or below the diagonal
@@ -306,7 +318,7 @@ k_simgemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
             const uint32_t acc = tile_iter & 1;
             mbar_wait(&acc_full[acc], (tile_iter >> 1) & 1);
             asm volatile("tcgen05.fence::after_thread_sync;" ::: "memory");
-            float* __restrict__ Sitem = S + (size_t)item * T * T;
+            float* __restrict__ Sitem = S + (size_t)item * rows * T;  // row-major rows [r0, row_end), pitch T
             const int row_base = m0 + quarter * 32;
 #pragma unroll 1
             for (int chunk = 0; chunk < BN / 32; ++chunk) {
@@ -330,7 +342,7 @@ k_simgemm(const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUt
 #pragma unroll 4
                     for (int r = 0; r < 32; ++r) {
                         const int row = row_base + r;
-                        if (row < T && (!crosses || col >= row)) Sitem[(size_t)row * T + col] = stage[r * EPI_PITCH + lane];
+                        if (row < row_end && (!crosses || col >= row)) Sitem[(size_t)(row - r0) * T + col] = stage[r * EPI_PITCH + lane];
                     }
                 }
                 __syncwarp();
@@ -374,22 +386,25 @@ bool make_map(CUtensorMap* map, const float* base, size_t rows, int box_rows) {
               CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE) == CUDA_SUCCESS;
 }
 
-template <int BN, bool SPLIT3>
-int launch_gemm(cudaStream_t st, const float* hi, const float* lo, int n_items, int T, float* S, int sm_count) {
+template <int BN, bool SPLIT3, bool TRI>
+int launch_gemm(cudaStream_t st, const float* hi, const float* lo, int n_items, int T, int r0, int rows, float* S,
+                int sm_count) {
     using Cfg = GemmCfg<BN, SPLIT3>;
     CUtensorMap map_a, map_b, map_a_lo, map_b_lo;
-    const size_t rows = (size_t)n_items * T;
-    if (!make_map(&map_a, hi, rows, BM) || !make_map(&map_b, hi, rows, BN)) return -1;
-    if (!make_map(&map_a_lo, SPLIT3 ? lo : hi, rows, BM) || !make_map(&map_b_lo, SPLIT3 ? lo : hi, rows, BN)) return -1;
+    const size_t op_rows = (size_t)n_items * T;
+    if (!make_map(&map_a, hi, op_rows, BM) || !make_map(&map_b, hi, op_rows, BN)) return -1;
+    if (!make_map(&map_a_lo, SPLIT3 ? lo : hi, op_rows, BM) || !make_map(&map_b_lo, SPLIT3 ? lo : hi, op_rows, BN)) return -1;
     static SmemOptIn opt_in;
     {
-        if (!smem_opt_in(k_simgemm<BN, SPLIT3>, (size_t)Cfg::SMEM, opt_in)) return -2;
+        if (!smem_opt_in(k_simgemm<BN, SPLIT3, TRI>, (size_t)Cfg::SMEM, opt_in)) return -2;
     }
-    const int mt = (T + BM - 1) / BM, nt = (T + BN - 1) / BN;
-    const int per_item = SPLIT3 ? triangle_tiles<BN / BM>(mt, nt) : mt * nt;
+    const int mt = (rows + BM - 1) / BM, nt = (T + BN - 1) / BN;
+    const int per_item = TRI ? triangle_tiles<BN / BM>(mt, nt) : mt * nt;
     const int tiles_total = n_items * per_item;
     const int grid = std::max(1, std::min(tiles_total, sm_count));
-    k_simgemm<BN, SPLIT3><<<grid, GEMM_THREADS, Cfg::SMEM, st>>>(map_a, map_b, map_a_lo, map_b_lo, T, n_items, per_item, S);
+    const int col_raster = rows < T ? 1 : 0;
+    k_simgemm<BN, SPLIT3, TRI><<<grid, GEMM_THREADS, Cfg::SMEM, st>>>(map_a, map_b, map_a_lo, map_b_lo, T, r0, rows, n_items,
+                                                                      per_item, col_raster, S);
     return 0;
 }
 
@@ -401,10 +416,22 @@ int launch_selfsim_tc(cudaStream_t st, const float* hi, const float* lo, int n_i
     // split product: 128 x 256 tiles (65 flop per operand byte from L2 instead of 49: the kernel runs at the L2
     // throughput cap, ncu profiles/r2a_sim); "simgemm_bn" = 128 selects the round-1 square tiles
     if (lo) {
-        if (g_tuning.simgemm_bn == 128) return launch_gemm<128, true>(st, hi, lo, n_items, T, S, sm_count);
-        return launch_gemm<256, true>(st, hi, lo, n_items, T, S, sm_count);
+        if (g_tuning.simgemm_bn == 128) return launch_gemm<128, true, true>(st, hi, lo, n_items, T, 0, T, S, sm_count);
+        return launch_gemm<256, true, true>(st, hi, lo, n_items, T, 0, T, S, sm_count);
     }
-    return launch_gemm<256, false>(st, hi, nullptr, n_items, T, S, sm_count);
+    return launch_gemm<256, false, false>(st, hi, nullptr, n_items, T, 0, T, S, sm_count);
+}
+
+// Row panel of one item: S_panel[r - r0][c] = <A[r], A[c]> for r in [r0, r0 + rows), c < T, row-major with pitch T.
+// The panel is a full rectangle (no mirror writes: S is not kept for later panels), so the split product costs twice
+// the MMAs per element of the triangle.  Tiles are rastered column by column.
+int launch_selfsim_tc_panel(cudaStream_t st, const float* hi, const float* lo, int T, int r0, int rows, float* S_panel,
+                            int sm_count) {
+    if (lo) {
+        if (g_tuning.simgemm_bn == 128) return launch_gemm<128, true, false>(st, hi, lo, 1, T, r0, rows, S_panel, sm_count);
+        return launch_gemm<256, true, false>(st, hi, lo, 1, T, r0, rows, S_panel, sm_count);
+    }
+    return launch_gemm<256, false, false>(st, hi, nullptr, 1, T, r0, rows, S_panel, sm_count);
 }
 
 }  // namespace repet

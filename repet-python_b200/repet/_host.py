@@ -64,6 +64,7 @@ SIGNATURES = {
     "repet_set_stream": (_c_int, [_vp, _vp]),
     "repet_set_window": (_c_int, [_vp, _vp, _c_int]),
     "repet_set_workspace_limit": (_c_int, [_vp, _c_u64]),
+    "repet_workspace_bytes": (_c_u64, [_vp]),
     "repet_synchronize": (_c_int, [_vp]),
     "repet_launch_count": (_c_u64, [_vp]),
     "repet_set_tuning": (_c_int, [ctypes.c_char_p, _c_int]),
@@ -215,6 +216,10 @@ class Handle:
 
     def set_workspace_limit(self, number_bytes):
         self.check(self.lib.repet_set_workspace_limit(self.h, int(number_bytes)))
+
+    def workspace_bytes(self):
+        """Bytes of device workspace the handle holds (grown on demand, kept between calls)."""
+        return int(self.lib.repet_workspace_bytes(self.h))
 
     def synchronize(self):
         self.check(self.lib.repet_synchronize(self.h))
