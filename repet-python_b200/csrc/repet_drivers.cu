@@ -38,6 +38,20 @@ struct PeriodShape {
     size_t bytes_per_item = 0;
 };
 
+// Workspace layouts.  Each carve is the single description of a pipeline's buffers for a chunk of g items: run on
+// Bump(nullptr) with g = 1 it gives the bytes per item the chunk sizes are computed from, and the runner carves the
+// same layout from its workspace.  Every take's count is affine in g with non-negative terms, so a layout for g
+// items never needs more than g x (its size for one item): a chunk of G = ws_bytes / bytes_per_item items fits.
+// A carve returns its buffers in a braced list, which is evaluated left to right: the members' order is the layout.
+struct PeriodBuffers { float2* X; float *P, *psd, *psd_im, *model; int* cert; double* cert_val; };
+
+PeriodBuffers carve_period(Bump& b, const PeriodShape& s, int nch, size_t g) {
+    const size_t psd_floats = g * s.n_blocks * s.n_parts * BEAT_L;
+    return {b.take<float2>(g * s.T * nch * XPITCH), b.take<float>(g * s.T * PPITCH), b.take<float>(psd_floats),
+            s.n_blocks > 1 ? b.take<float>(psd_floats) : nullptr, b.take<float>(g * nch * s.pmax * PPITCH),
+            b.take<int>(g * (CERT_MAX + 1)), b.take<double>(g * CERT_MAX * CERT_TSPLIT)};  // period certification
+}
+
 void pick_beat_parts(repet_handle* h, int chunk_hint, int floor_parts, int* n_parts, int* f_per_part) {
     // measured on B200 (profiles/r1_sweep2.txt): ~64 partitions of the 1025 rows per clip is the sweet spot
     int want = std::max(floor_parts, std::min(129, (h->sm_count * 6 + chunk_hint - 1) / std::max(1, chunk_hint)));
@@ -64,13 +78,9 @@ int period_shape(repet_handle* h, const repet_params* p, int nch, int64_t n_samp
         s->n_blocks = (T + s->block_frames - 1) / s->block_frames;
     }
     pick_beat_parts(h, chunk_hint * s->n_blocks, s->n_blocks > 1 ? 16 : 64, &s->n_parts, &s->f_per_part);
-    size_t b = 0;
-    b += align_up((size_t)T * nch * XPITCH * sizeof(float2));
-    b += align_up((size_t)T * PPITCH * sizeof(float));
-    b += (s->n_blocks > 1 ? 2 : 1) * align_up((size_t)s->n_blocks * s->n_parts * BEAT_L * sizeof(float));
-    b += align_up((size_t)nch * s->pmax * PPITCH * sizeof(float));
-    b += 2048;  // period certification records
-    s->bytes_per_item = b;
+    Bump measure(nullptr);
+    carve_period(measure, *s, nch, 1);
+    s->bytes_per_item = measure.off;
     return REPET_OK;
 }
 
@@ -85,23 +95,19 @@ int period_pipeline(repet_handle* h, const float* audio, Geom gin, float* out, G
                     const repet_params* p, const PeriodShape& s, int32_t* periods_dev, unsigned char* ws,
                     size_t ws_bytes) {
     const int n_items = gin.n_items;
+    // carve_period(g) <= g x bytes_per_item (see the layouts above)
     const int G = (int)std::min<size_t>(std::min<size_t>((size_t)n_items, MAX_ITEMS_PER_LAUNCH),
                                         std::max<size_t>(1, ws_bytes / s.bytes_per_item));
     const float scale = (float)(1.0 / ((double)WIN_N * p->cola_gain));
     cudaStream_t st = h->stream;
+    const bool blocked = s.n_blocks > 1;
+    const int beat_L = blocked ? BEAT_L : beat_transform_length(s.T, s.lag_hi);
+    const int total_parts = s.n_blocks * s.n_parts;
     for (int first = 0; first < n_items; first += G) {
         const int g_items = std::min(G, n_items - first);
-        Bump bump(ws);
-        float2* X = bump.take<float2>((size_t)g_items * s.T * nch * XPITCH);
-        float* P = bump.take<float>((size_t)g_items * s.T * PPITCH);
-        const bool blocked = s.n_blocks > 1;
-        const int beat_L = blocked ? BEAT_L : beat_transform_length(s.T, s.lag_hi);
-        const int total_parts = s.n_blocks * s.n_parts;
-        float* psd = bump.take<float>((size_t)g_items * total_parts * BEAT_L);
-        float* psd_im = blocked ? bump.take<float>((size_t)g_items * total_parts * BEAT_L) : nullptr;
-        float* model = bump.take<float>((size_t)g_items * nch * s.pmax * PPITCH);
-        int* cert = bump.take<int>((size_t)g_items * (CERT_MAX + 1));
-        double* cert_val = bump.take<double>((size_t)g_items * CERT_MAX * 16);  // x CERT_TSPLIT partial sums
+        Bump bump(ws, ws_bytes);
+        const auto [X, P, psd, psd_im, model, cert, cert_val] = carve_period(bump, s, nch, g_items);
+        if (!bump.fits()) return fail(h, REPET_E_CUDA, "period pipeline layout exceeds its workspace");
         gin.n_items = gout.n_items = g_items;
         gin.item0 = gout.item0 = first;
         const int K = pick_frames_per_cta(h, (long long)g_items * s.T);
@@ -174,6 +180,44 @@ struct Plan {
     size_t bytes_per_clip = 0;
 };
 
+// extended: the segments' backgrounds and periods; the period pipeline of the segments runs in what follows them
+struct ExtendedBuffers { float *seg_main, *seg_last; int32_t *per_main, *per_last; };
+
+ExtendedBuffers carve_extended(Bump& b, const Plan& plan, size_t g) {
+    const size_t n_main = plan.n_seg - 1;
+    return {b.take<float>(g * n_main * plan.nch * plan.seg_len), b.take<float>(g * plan.nch * plan.last_len),
+            b.take<int32_t>(g * n_main), b.take<int32_t>(g)};
+}
+
+struct AdaptiveBuffers { float2* X; float *P, *psd; int32_t* seg_period; float *model, *Vsq; int* cert; double* cert_val; };
+
+AdaptiveBuffers carve_adaptive(Bump& b, const Plan& plan, size_t g) {
+    const size_t T = plan.T, items = g * plan.n_beat_seg, planes = g * plan.nch * T * PPITCH;
+    return {b.take<float2>(g * T * plan.nch * XPITCH), b.take<float>(g * T * PPITCH),
+            b.take<float>(items * plan.beat_parts * BEAT_L), b.take<int32_t>(items),
+            b.take<float>(planes), g_tuning.adaptive_vsq ? b.take<float>(planes) : nullptr,  // model, squared magnitudes
+            b.take<int>(items * (CERT_MAX + 1)), b.take<double>(items * CERT_MAX * CERT_TSPLIT)};  // period certification
+}
+
+// sim / simonline; `s_floats` is the size of the similarity matrix S (sim only): g whole matrices or one row panel
+struct SimBuffers {
+    float2* X; float* V; double* An64; int32_t *idx, *cnt; float *model, *Vsq; int32_t* overflow;
+    float *An32, *An32lo, *S; int32_t* ovf_cols; unsigned char* ovf_scratch;
+};
+
+SimBuffers carve_sim(Bump& b, const Plan& plan, size_t g, size_t s_floats, int sm_count) {
+    const size_t T = plan.T, planes = g * plan.nch * T * PPITCH;
+    const bool sim = plan.kind == KIND_SIM;
+    return {b.take<float2>(g * T * plan.nch * XPITCH), b.take<float>(g * T * PPITCH), b.take<double>(g * T * APITCH64),
+            b.take<int32_t>(g * T * plan.number), b.take<int32_t>(g * T),  // idx, cnt
+            b.take<float>(planes), plan.number > 32 ? b.take<float>(planes) : nullptr,  // model, squared magnitudes
+            b.take<int32_t>(4),  // [overflow flag, candidates, uncertain, neighbour dots]
+            sim ? b.take<float>(g * T * KPAD) : nullptr, sim ? b.take<float>(g * T * KPAD) : nullptr,  // An32 hi, lo
+            sim ? b.take<float>(s_floats) : nullptr,
+            sim ? b.take<int32_t>(g * T) : nullptr,  // columns handed to the exact fallback
+            sim ? b.take<unsigned char>(topk_exact_scratch_bytes(plan.T, sm_count)) : nullptr};
+}
+
 int make_plan(repet_handle* h, int kind, const repet_params* p, int nch, int64_t S, int chunk_hint, Plan* plan) {
     plan->kind = kind;
     plan->nch = nch;
@@ -207,12 +251,10 @@ int make_plan(repet_handle* h, int kind, const repet_params* p, int nch, int64_t
         if ((rc = period_shape(h, p, nch, seg_len, main_hint, &plan->seg_main))) return rc;
         if ((rc = period_shape(h, p, nch, plan->last_len, chunk_hint, &plan->seg_last))) return rc;
         plan->ints_per_clip = plan->n_seg;
-        size_t b = 0;
-        b += align_up((size_t)(plan->n_seg - 1) * nch * seg_len * sizeof(float));
-        b += align_up((size_t)nch * plan->last_len * sizeof(float));
-        b += (size_t)(plan->n_seg - 1) * plan->seg_main.bytes_per_item + plan->seg_last.bytes_per_item;
-        b += 1024;
-        plan->bytes_per_clip = b;
+        Bump measure(nullptr);
+        carve_extended(measure, *plan, 1);
+        plan->bytes_per_clip = measure.off + (size_t)(plan->n_seg - 1) * plan->seg_main.bytes_per_item +
+                               plan->seg_last.bytes_per_item;
         return REPET_OK;
     }
     if (kind == KIND_ADAPTIVE) {
@@ -231,17 +273,9 @@ int make_plan(repet_handle* h, int kind, const repet_params* p, int nch, int64_t
         plan->n_beat_seg = (plan->T + step - 1) / step;
         pick_beat_parts(h, chunk_hint * plan->n_beat_seg, 4, &plan->beat_parts, &plan->beat_f_per_part);
         plan->ints_per_clip = plan->T;
-        size_t b = 0;
-        b += align_up((size_t)plan->T * nch * XPITCH * sizeof(float2));
-        b += align_up((size_t)plan->T * PPITCH * sizeof(float));
-        b += align_up((size_t)plan->n_beat_seg * plan->beat_parts * BEAT_L * sizeof(float));
-        b += align_up((size_t)plan->n_beat_seg * sizeof(int32_t));
-        b += align_up((size_t)nch * plan->T * PPITCH * sizeof(float));
-        b += align_up((size_t)nch * plan->T * PPITCH * sizeof(float));               // squared magnitudes (adaptive_vsq)
-        b += align_up((size_t)plan->n_beat_seg * (CERT_MAX + 1) * sizeof(int));       // period certification records
-        b += align_up((size_t)plan->n_beat_seg * CERT_MAX * 16 * sizeof(double));
-        b += 1024;
-        plan->bytes_per_clip = b;
+        Bump measure(nullptr);
+        carve_adaptive(measure, *plan, 1);
+        plan->bytes_per_clip = measure.off;
         return REPET_OK;
     }
     if (kind == KIND_SIM || kind == KIND_SIMONLINE) {
@@ -264,37 +298,23 @@ int make_plan(repet_handle* h, int kind, const repet_params* p, int nch, int64_t
             plan->buffer_frames = B;
         }
         plan->ints_per_clip = T * (plan->number + 1);
-        size_t b = 0;
-        b += align_up((size_t)T * nch * XPITCH * sizeof(float2));   // X
-        b += align_up((size_t)T * PPITCH * sizeof(float));          // V = mean_c |X|
-        b += align_up((size_t)T * APITCH64 * sizeof(double));       // An64
-        b += align_up((size_t)T * plan->number * sizeof(int32_t));  // idx
-        b += align_up((size_t)T * sizeof(int32_t));                 // cnt
-        b += align_up((size_t)nch * T * PPITCH * sizeof(float));    // model
-        if (plan->number > 32) b += align_up((size_t)nch * T * PPITCH * sizeof(float));  // squared magnitudes
+        auto clip_bytes = [&](size_t s_floats) { Bump m(nullptr); carve_sim(m, *plan, 1, s_floats, h->sm_count); return m.off; };
+        size_t s_floats = 0;  // simonline forms no S
         if (kind == KIND_SIM) {
-            b += 2 * align_up((size_t)T * KPAD * sizeof(float));  // An32 hi, lo
-            b += align_up((size_t)T * sizeof(int32_t));       // columns handed to the exact fallback
-            b += align_up(topk_exact_scratch_bytes(T, h->sm_count));
-            b += 2048;
-            // S: the whole matrix when it fits the workspace limit with the linear part above; otherwise row panels
-            // of as many rows as the limit leaves room for (128 when the linear part alone exceeds it), one track
-            // per chunk
-            const size_t row_bytes = (size_t)T * sizeof(float);
-            const size_t whole = align_up((size_t)T * row_bytes);
+            // S: the whole matrix when it fits the workspace limit beside the linear part; otherwise row panels of
+            // as many rows as the limit leaves room for (128 when the linear part alone exceeds it), one track per
+            // chunk
+            const size_t linear = clip_bytes(0), row_bytes = (size_t)T * sizeof(float);
             const size_t limit = default_ws_limit(h);
             plan->panel_rows = 0;
-            if (b + whole > limit) {
-                const size_t room = limit > b + 256 ? (limit - b - 256) / row_bytes : 0;
+            if (clip_bytes((size_t)T * T) > limit) {
+                const size_t room = limit > linear + 256 ? (limit - linear - 256) / row_bytes : 0;  // 256: alignment
                 const int P = (int)std::max<size_t>(128, std::min<size_t>(room, (size_t)T) / 128 * 128);
                 if (P < T) plan->panel_rows = P;
             }
-            b += plan->panel_rows ? align_up((size_t)plan->panel_rows * row_bytes) : whole;
-            plan->bytes_per_clip = b;
-            return REPET_OK;
+            s_floats = (size_t)(plan->panel_rows ? plan->panel_rows : T) * T;
         }
-        b += 2048;
-        plan->bytes_per_clip = b;
+        plan->bytes_per_clip = clip_bytes(s_floats);
         return REPET_OK;
     }
     return fail(h, REPET_E_INVALID_ARG, "unknown driver kind");
@@ -316,27 +336,18 @@ int run_sim(repet_handle* h, const Plan& plan, const float* audio, int n_clips, 
     const int nch = plan.nch, T = plan.T;
     const bool online = plan.kind == KIND_SIMONLINE;
     const int P = online ? 0 : plan.panel_rows;  // row panels: one track per chunk
+    // carve_sim(g) <= g x bytes_per_clip (see the layouts above)
     const int G = P ? 1 : (int)std::min<size_t>(std::min<size_t>((size_t)n_clips, MAX_ITEMS_PER_LAUNCH / 2),
                                                 std::max<size_t>(1, ws_bytes / plan.bytes_per_clip));
     const float scale = (float)(1.0 / ((double)WIN_N * plan.p.cola_gain));
+    const int fast = g_tuning.simgemm_tc;
     cudaStream_t st = h->stream;
     for (int clip0 = 0; clip0 < n_clips; clip0 += G) {
         const int g = std::min(G, n_clips - clip0);
-        Bump bump(ws);
-        float2* X = bump.take<float2>((size_t)g * T * nch * XPITCH);
-        float* V = bump.take<float>((size_t)g * T * PPITCH);
-        double* An64 = bump.take<double>((size_t)g * T * APITCH64);
-        int32_t* idx = bump.take<int32_t>((size_t)g * T * plan.number);
-        int32_t* cnt = bump.take<int32_t>((size_t)g * T);
-        float* model = bump.take<float>((size_t)g * nch * T * PPITCH);
-        float* Vsq = plan.number > 32 ? bump.take<float>((size_t)g * nch * T * PPITCH) : nullptr;
-        int32_t* overflow = bump.take<int32_t>(4);  // [overflow flag, candidates, uncertain, neighbour dots]
-        float* An32 = online ? nullptr : bump.take<float>((size_t)g * T * KPAD);
-        float* An32lo = online ? nullptr : bump.take<float>((size_t)g * T * KPAD);
-        const int fast = g_tuning.simgemm_tc;
-        float* S = online ? nullptr : bump.take<float>(P ? (size_t)P * T : (size_t)g * T * T);
-        int32_t* ovf_cols = online ? nullptr : bump.take<int32_t>((size_t)g * T);
-        unsigned char* ovf_scratch = online ? nullptr : bump.take<unsigned char>(topk_exact_scratch_bytes(T, h->sm_count));
+        Bump bump(ws, ws_bytes);
+        const auto [X, V, An64, idx, cnt, model, Vsq, overflow, An32, An32lo, S, ovf_cols, ovf_scratch] =
+            carve_sim(bump, plan, g, (P ? (size_t)P : (size_t)g * T) * T, h->sm_count);
+        if (!bump.fits()) return fail(h, REPET_E_CUDA, "sim layout exceeds its workspace");
         Geom geom = clip_geom(g, nch, plan.S, T);
         geom.first_offset = (long long)clip0 * geom.clip_stride;
         if (online) {
@@ -369,47 +380,30 @@ int run_sim(repet_handle* h, const Plan& plan, const float* audio, int n_clips, 
         } else {
             const float tau = fast >= 2 ? TAU_3XTF32_GEMM : (fast ? TAU_TF32_GEMM : TAU_FP32_GEMM);
             const double thr = plan.p.similarity_threshold;
-            if (!P) {
+            const float* lo = fast >= 2 ? An32lo : nullptr;
+            // rows [r0, r0 + rows) of S, then the columns they settle: one range covers the whole matrices of the g
+            // tracks (the GEMM forms their upper triangles), or ranges of P rows cover one track panel by panel.  The
+            // columns k_topk queues for the exact fallback accumulate over the ranges and are settled once at the end
+            CU(cudaMemsetAsync(overflow, 0, 4 * sizeof(int32_t), st));
+            const int range = P ? P : T;
+            for (int r0 = 0; r0 < T; r0 += range) {
+                const int rows = std::min(range, T - r0);
                 {
                     Timed timed(h, REPET_K_SIMGEMM);
-                    if (fast) {
-                        if (launch_selfsim_tc(st, An32, fast >= 2 ? An32lo : nullptr, g, T, S, h->sm_count))
-                            return fail(h, REPET_E_CUDA, "tensor-map encode failed for the similarity GEMM");
-                    } else {
-                        launch_selfsim_simt(st, An32, g, T, S);
-                    }
-                }
-                CU(cudaMemsetAsync(overflow, 0, 4 * sizeof(int32_t), st));
-                Timed timed(h, REPET_K_TOPK, 2);  // k_topk, k_topk_exact
-                if (launch_topk_propose(st, S, 0, T, An64, g, T, tau, thr, plan.distance, plan.number, idx, cnt, overflow,
-                                        ovf_cols))
-                    return fail(h, REPET_E_UNSUPPORTED, "similarity_distance too large for the in-shared-memory similarity row");
-                launch_topk_exact(st, An64, T, thr, plan.distance, plan.number, overflow, ovf_cols, ovf_scratch, idx, cnt,
-                                  h->sm_count);
-            } else {
-                // rows [r0, r0 + P) of S, then the columns they settle; the columns k_topk queues for the exact
-                // fallback accumulate over the panels and are settled once at the end
-                CU(cudaMemsetAsync(overflow, 0, 4 * sizeof(int32_t), st));
-                for (int r0 = 0; r0 < T; r0 += P) {
-                    const int rows = std::min(P, T - r0);
-                    {
-                        Timed timed(h, REPET_K_SIMGEMM);
-                        if (fast) {
-                            if (launch_selfsim_tc_panel(st, An32, fast >= 2 ? An32lo : nullptr, T, r0, rows, S, h->sm_count))
-                                return fail(h, REPET_E_CUDA, "tensor-map encode failed for the similarity GEMM");
-                        } else {
-                            launch_selfsim_simt_panel(st, An32, T, r0, rows, S);
-                        }
-                    }
-                    Timed timed(h, REPET_K_TOPK);
-                    if (launch_topk_propose(st, S, r0, rows, An64, 1, T, tau, thr, plan.distance, plan.number, idx, cnt,
-                                            overflow, ovf_cols))
-                        return fail(h, REPET_E_UNSUPPORTED, "similarity_distance too large for the in-shared-memory similarity row");
+                    if (!fast)
+                        P ? launch_selfsim_simt_panel(st, An32, T, r0, rows, S) : launch_selfsim_simt(st, An32, g, T, S);
+                    else if (P ? launch_selfsim_tc_panel(st, An32, lo, T, r0, rows, S, h->sm_count)
+                               : launch_selfsim_tc(st, An32, lo, g, T, S, h->sm_count))
+                        return fail(h, REPET_E_CUDA, "tensor-map encode failed for the similarity GEMM");
                 }
                 Timed timed(h, REPET_K_TOPK);
-                launch_topk_exact(st, An64, T, thr, plan.distance, plan.number, overflow, ovf_cols, ovf_scratch, idx, cnt,
-                                  h->sm_count);
+                if (launch_topk_propose(st, S, r0, rows, An64, g, T, tau, thr, plan.distance, plan.number, idx, cnt,
+                                        overflow, ovf_cols))
+                    return fail(h, REPET_E_UNSUPPORTED, "similarity_distance too large for the in-shared-memory similarity row");
             }
+            Timed timed(h, REPET_K_TOPK);
+            launch_topk_exact(st, An64, T, thr, plan.distance, plan.number, overflow, ovf_cols, ovf_scratch, idx, cnt,
+                              h->sm_count);
         }
         {
             Timed timed(h, REPET_K_MODEL, Vsq ? 3 : 2);  // k_simmodel, [k_simmodel_large,] k_simmodel_nyquist
@@ -439,15 +433,14 @@ int run_extended(repet_handle* h, const Plan& plan, const float* audio, int n_cl
                  unsigned char* ws, size_t ws_bytes) {
     const int nch = plan.nch;
     const int n_main = plan.n_seg - 1;
+    // carve_extended(g) plus the period layouts of its g x n_seg segments <= g x bytes_per_clip (see the layouts above)
     const int G = (int)std::min<size_t>((size_t)n_clips, std::max<size_t>(1, ws_bytes / plan.bytes_per_clip));
     cudaStream_t st = h->stream;
     for (int clip0 = 0; clip0 < n_clips; clip0 += G) {
         const int g = std::min(G, n_clips - clip0);
-        Bump bump(ws);
-        float* seg_main = bump.take<float>((size_t)g * n_main * nch * plan.seg_len);
-        float* seg_last = bump.take<float>((size_t)g * nch * plan.last_len);
-        int32_t* per_main = bump.take<int32_t>((size_t)g * n_main);
-        int32_t* per_last = bump.take<int32_t>((size_t)g);
+        Bump bump(ws, ws_bytes);
+        const auto [seg_main, seg_last, per_main, per_last] = carve_extended(bump, plan, g);
+        if (!bump.fits()) return fail(h, REPET_E_CUDA, "extended layout exceeds its workspace");
         unsigned char* pws = ws + bump.off;
         const size_t pws_bytes = ws_bytes - bump.off;
         const float* a = audio + (size_t)clip0 * nch * plan.S;
@@ -486,21 +479,16 @@ int run_adaptive(repet_handle* h, const Plan& plan, const float* audio, int n_cl
     const int nch = plan.nch, T = plan.T;
     // grid.y carries clips x beat segments in k_beat: keep it below 65535
     const size_t grid_cap = std::max<size_t>(1, 60000 / (size_t)std::max(1, plan.n_beat_seg));
+    // carve_adaptive(g) <= g x bytes_per_clip (see the layouts above)
     const int G = (int)std::min<size_t>(std::min<size_t>((size_t)n_clips, std::min<size_t>(MAX_ITEMS_PER_LAUNCH / 2, grid_cap)),
                                         std::max<size_t>(1, ws_bytes / plan.bytes_per_clip));
     const float scale = (float)(1.0 / ((double)WIN_N * plan.p.cola_gain));
     cudaStream_t st = h->stream;
     for (int clip0 = 0; clip0 < n_clips; clip0 += G) {
         const int g = std::min(G, n_clips - clip0);
-        Bump bump(ws);
-        float2* X = bump.take<float2>((size_t)g * T * nch * XPITCH);
-        float* P = bump.take<float>((size_t)g * T * PPITCH);
-        float* psd = bump.take<float>((size_t)g * plan.n_beat_seg * plan.beat_parts * BEAT_L);
-        int32_t* seg_period = bump.take<int32_t>((size_t)g * plan.n_beat_seg);
-        float* model = bump.take<float>((size_t)g * nch * T * PPITCH);
-        float* Vsq = g_tuning.adaptive_vsq ? bump.take<float>((size_t)g * nch * T * PPITCH) : nullptr;
-        int* cert = bump.take<int>((size_t)g * plan.n_beat_seg * (CERT_MAX + 1));
-        double* cert_val = bump.take<double>((size_t)g * plan.n_beat_seg * CERT_MAX * 16);  // x CERT_TSPLIT partial sums
+        Bump bump(ws, ws_bytes);
+        const auto [X, P, psd, seg_period, model, Vsq, cert, cert_val] = carve_adaptive(bump, plan, g);
+        if (!bump.fits()) return fail(h, REPET_E_CUDA, "adaptive layout exceeds its workspace");
         int32_t* frame_period = ints + (size_t)clip0 * T;
         Geom geom = clip_geom(g, nch, plan.S, T);
         geom.first_offset = (long long)clip0 * geom.clip_stride;
@@ -571,10 +559,14 @@ int batch_dev(repet_handle* h, int kind, const float* audio, int n_clips, int nc
     if (ints_per_clip_out) *ints_per_clip_out = plan.ints_per_clip;
     if (n_clips == 0) return REPET_OK;
     G = chunk_clips(h, plan, n_clips);
-    const size_t ints_bytes = ints_dev ? 0 : align_up((size_t)n_clips * plan.ints_per_clip * sizeof(int32_t));
-    if ((rc = ensure_arena(h, ints_bytes + (size_t)G * plan.bytes_per_clip))) return rc;
-    int32_t* ints = ints_dev ? ints_dev : reinterpret_cast<int32_t*>(h->arena);
-    rc = run_plan(h, plan, audio, n_clips, background, ints, h->arena + ints_bytes, (size_t)G * plan.bytes_per_clip);
+    const size_t ws_bytes = (size_t)G * plan.bytes_per_clip;
+    int32_t* ints = ints_dev; unsigned char* ws;
+    rc = carve_arena(h, [&](Bump& b) {
+        if (!ints_dev) ints = b.take<int32_t>((size_t)n_clips * plan.ints_per_clip);
+        ws = b.take<unsigned char>(ws_bytes);
+    });
+    if (rc) return rc;
+    rc = run_plan(h, plan, audio, n_clips, background, ints, ws, ws_bytes);
     if (rc) return rc;
     if (ints_host) {
         CU(cudaMemcpyAsync(ints_host, ints, (size_t)n_clips * plan.ints_per_clip * sizeof(int32_t), cudaMemcpyDeviceToHost,
@@ -614,20 +606,17 @@ int batch_host(repet_handle* h, int kind, const void* audio_any, int in_fmt, int
     Plan plan;
     if ((rc = make_plan(h, kind, p, nch, S, Gc, &plan))) return rc;
     const int Gw = std::min(Gc, chunk_clips(h, plan, Gc));
-    const size_t in_slot_bytes = align_up((size_t)Gc * in_clip_bytes), out_slot_bytes = align_up((size_t)Gc * out_clip_bytes);
-    const size_t f32_bytes = align_up((size_t)Gc * clip_bytes);
-    const size_t ints_bytes = align_up((size_t)n_clips * plan.ints_per_clip * sizeof(int32_t));
     const size_t ws_bytes = (size_t)Gw * plan.bytes_per_clip;
-    if ((rc = ensure_arena(h, ints_bytes + 2 * in_slot_bytes + 2 * out_slot_bytes + (pcm_in ? f32_bytes : 0) +
-                                  (pcm_out ? f32_bytes : 0) + ws_bytes)))
-        return rc;
-    Bump bump(h->arena);
-    int32_t* ints = reinterpret_cast<int32_t*>(bump.take<unsigned char>(ints_bytes));
-    unsigned char* in_slot[2] = {bump.take<unsigned char>(in_slot_bytes), bump.take<unsigned char>(in_slot_bytes)};
-    unsigned char* out_slot[2] = {bump.take<unsigned char>(out_slot_bytes), bump.take<unsigned char>(out_slot_bytes)};
-    float* in32 = pcm_in ? reinterpret_cast<float*>(bump.take<unsigned char>(f32_bytes)) : nullptr;
-    float* out32 = pcm_out ? reinterpret_cast<float*>(bump.take<unsigned char>(f32_bytes)) : nullptr;
-    unsigned char* ws = h->arena + bump.off;
+    int32_t* ints; unsigned char *in_slot[2], *out_slot[2], *ws; float *in32 = nullptr, *out32 = nullptr;
+    rc = carve_arena(h, [&](Bump& b) {
+        ints = b.take<int32_t>((size_t)n_clips * plan.ints_per_clip);
+        for (unsigned char*& slot : in_slot) slot = b.take<unsigned char>((size_t)Gc * in_clip_bytes);
+        for (unsigned char*& slot : out_slot) slot = b.take<unsigned char>((size_t)Gc * out_clip_bytes);
+        if (pcm_in) in32 = b.take<float>((size_t)Gc * clip_elems);
+        if (pcm_out) out32 = b.take<float>((size_t)Gc * clip_elems);
+        ws = b.take<unsigned char>(ws_bytes);
+    });
+    if (rc) return rc;
     CU(cudaStreamSynchronize(h->stream));  // the arena must be idle before the copy streams touch it
     auto pipeline = [&]() -> int {
         int n_chunks = 0;
@@ -715,17 +704,17 @@ int single_f64(repet_handle* h, int kind, const double* audio, int64_t S, int nc
     const size_t n = (size_t)S * nch;
     const int T_spec = frames_of(S);
     const size_t spec_elems = spectrograms ? (size_t)3 * T_spec * PPITCH : 0;
-    const size_t need = align_up((size_t)plan.ints_per_clip * sizeof(int32_t)) + align_up(n * sizeof(double)) +
-                        3 * align_up(n * sizeof(float)) + align_up(spec_elems * sizeof(float)) + plan.bytes_per_clip;
-    if ((rc = ensure_arena(h, need))) return rc;
-    Bump bump(h->arena);
-    int32_t* ints = bump.take<int32_t>(plan.ints_per_clip);
-    double* d64 = bump.take<double>(n);
-    float* in32 = bump.take<float>(n);
-    float* out32 = bump.take<float>(n);
-    float* fg32 = bump.take<float>(n);
-    float* spec = bump.take<float>(spec_elems);
-    unsigned char* ws = h->arena + bump.off;
+    int32_t* ints; double* d64; float *in32, *out32, *fg32, *spec; unsigned char* ws;
+    rc = carve_arena(h, [&](Bump& b) {
+        ints = b.take<int32_t>(plan.ints_per_clip);
+        d64 = b.take<double>(n);
+        in32 = b.take<float>(n);
+        out32 = b.take<float>(n);
+        fg32 = b.take<float>(n);
+        spec = b.take<float>(spec_elems);
+        ws = b.take<unsigned char>(plan.bytes_per_clip);
+    });
+    if (rc) return rc;
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(d64, audio, n * sizeof(double), cudaMemcpyHostToDevice, st));
     {
@@ -774,14 +763,14 @@ int single_f64_dev(repet_handle* h, int kind, const double* d_audio, int64_t S, 
     Plan plan;
     if ((rc = make_plan(h, kind, p, nch, S, 1, &plan))) return rc;
     const size_t n = (size_t)S * nch;
-    const size_t need = align_up((size_t)plan.ints_per_clip * sizeof(int32_t)) + 2 * align_up(n * sizeof(float)) +
-                        plan.bytes_per_clip;
-    if ((rc = ensure_arena(h, need))) return rc;
-    Bump bump(h->arena);
-    int32_t* ints = bump.take<int32_t>(plan.ints_per_clip);
-    float* in32 = bump.take<float>(n);
-    float* out32 = bump.take<float>(n);
-    unsigned char* ws = h->arena + bump.off;
+    int32_t* ints; float *in32, *out32; unsigned char* ws;
+    rc = carve_arena(h, [&](Bump& b) {
+        ints = b.take<int32_t>(plan.ints_per_clip);
+        in32 = b.take<float>(n);
+        out32 = b.take<float>(n);
+        ws = b.take<unsigned char>(plan.bytes_per_clip);
+    });
+    if (rc) return rc;
     cudaStream_t st = h->stream;
     {
         Timed timed(h, REPET_K_CONVERT);

@@ -14,8 +14,8 @@
 namespace {
 
 using repet::fail;
-using repet::align_up;
 using repet::Bump;
+using repet::carve_arena;
 
 __device__ __forceinline__ double2 zmul(double2 a, double2 b) {
     return make_double2(fma(a.x, b.x, -a.y * b.y), fma(a.x, b.y, a.y * b.x));
@@ -241,13 +241,11 @@ __global__ void k_scale_beat(double* __restrict__ beat, int n, int n_seq) {
     if (l < n) beat[l] /= (double)n_seq;
 }
 
-int acorr_device(repet_handle* h, const double* d_data, int n_rows, int n_cols, double* d_out, unsigned char* ws) {
+// z, tmp: [n_cols][L] each, L = next_pow2(2 n_rows)
+int acorr_device(repet_handle* h, const double* d_data, int n_rows, int n_cols, double* d_out, double2* z, double2* tmp) {
     // any L >= 2 n_rows - 1 gives the same linear autocorrelation as the reference's length 2 n_rows (quirk Q13)
     const int L = next_pow2(2LL * n_rows);
     cudaStream_t st = h->stream;
-    Bump bump(ws);
-    double2* z = bump.take<double2>((size_t)n_cols * L);
-    double2* tmp = bump.take<double2>((size_t)n_cols * L);
     const long long total = (long long)n_cols * L;
     k_load_columns<<<(unsigned)((total + 255) / 256), 256, 0, st>>>(d_data, n_rows, n_cols, L, z);
     fft_pow2(st, z, tmp, L, n_cols, false);
@@ -283,16 +281,15 @@ int repet_stft_f64(repet_handle* h, const double* signal, int64_t n_samples, con
     if (T < 1) return fail(h, REPET_E_INVALID_ARG, "signal too short for one frame");
     CU(cudaSetDevice(h->device));
     const size_t elems = (size_t)T * N;
-    const size_t need = align_up((size_t)std::max<int64_t>(n_samples, 1) * sizeof(double)) + align_up((size_t)N * sizeof(double)) +
-                        2 * align_up(elems * sizeof(double2)) + align_up(fft_any_workspace(N, T) * sizeof(double2)) + 1024;
-    int rc = repet::ensure_arena(h, need);
+    double *d_sig, *d_win; double2 *frames, *out, *ws;
+    int rc = carve_arena(h, [&](Bump& b) {
+        d_sig = b.take<double>((size_t)std::max<int64_t>(n_samples, 1));
+        d_win = b.take<double>(N);
+        frames = b.take<double2>(elems);
+        out = b.take<double2>(elems);
+        ws = b.take<double2>(fft_any_workspace(N, T));
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    double* d_sig = bump.take<double>((size_t)std::max<int64_t>(n_samples, 1));
-    double* d_win = bump.take<double>(N);
-    double2* frames = bump.take<double2>(elems);
-    double2* out = bump.take<double2>(elems);
-    double2* ws = bump.take<double2>(fft_any_workspace(N, T));
     cudaStream_t st = h->stream;
     if (n_samples > 0) CU(cudaMemcpyAsync(d_sig, signal, (size_t)n_samples * sizeof(double), cudaMemcpyHostToDevice, st));
     CU(cudaMemcpyAsync(d_win, window, (size_t)N * sizeof(double), cudaMemcpyHostToDevice, st));
@@ -321,15 +318,14 @@ int repet_istft_f64(repet_handle* h, const double* spectrum, int window_length, 
     for (int i = 0; i < N; i += step_length) gain += window[i];  // sum(window[0:N:step]), repet.py:1103
     CU(cudaSetDevice(h->device));
     const size_t elems = (size_t)T * N;
-    const size_t need = 2 * align_up(elems * sizeof(double2)) + align_up(fft_any_workspace(N, T) * sizeof(double2)) +
-                        align_up((size_t)n_out * sizeof(double)) + 1024;
-    int rc = repet::ensure_arena(h, need);
+    double2 *in, *frames, *ws; double* out;
+    int rc = carve_arena(h, [&](Bump& b) {
+        in = b.take<double2>(elems);
+        frames = b.take<double2>(elems);
+        ws = b.take<double2>(fft_any_workspace(N, T));
+        out = b.take<double>((size_t)n_out);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    double2* in = bump.take<double2>(elems);
-    double2* frames = bump.take<double2>(elems);
-    double2* ws = bump.take<double2>(fft_any_workspace(N, T));
-    double* out = bump.take<double>((size_t)n_out);
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(in, spectrum, elems * sizeof(double2), cudaMemcpyHostToDevice, st));
     transpose(st, in, N, (int)T, frames);  // (N, T) -> [T][N]
@@ -350,26 +346,26 @@ int repet_acorr_f64(repet_handle* h, const double* data, int n_rows, int n_colum
     const size_t n = (size_t)n_rows * n_columns;
     // columns in chunks so that the two transform buffers stay below ~4 GB
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_columns, ((size_t)2 << 30) / ((size_t)L * sizeof(double2))));
-    const size_t need = 2 * align_up(n * sizeof(double)) + 2 * align_up((size_t)chunk * L * sizeof(double2)) +
-                        2 * align_up((size_t)n_rows * chunk * sizeof(double)) + 1024;
-    int rc = repet::ensure_arena(h, need);
+    double *d_in, *d_out, *c_in, *c_out; double2 *z, *tmp;
+    int rc = carve_arena(h, [&](Bump& b) {
+        d_in = b.take<double>(n);
+        d_out = b.take<double>(n);
+        c_in = b.take<double>((size_t)n_rows * chunk);
+        c_out = b.take<double>((size_t)n_rows * chunk);
+        z = b.take<double2>((size_t)chunk * L);
+        tmp = b.take<double2>((size_t)chunk * L);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    double* d_in = bump.take<double>(n);
-    double* d_out = bump.take<double>(n);
-    double* c_in = bump.take<double>((size_t)n_rows * chunk);
-    double* c_out = bump.take<double>((size_t)n_rows * chunk);
-    unsigned char* ws = h->arena + bump.off;
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(d_in, data, n * sizeof(double), cudaMemcpyHostToDevice, st));
     for (int c0 = 0; c0 < n_columns; c0 += chunk) {
         const int g = std::min(chunk, n_columns - c0);
         if (g == n_columns) {
-            if ((rc = acorr_device(h, d_in, n_rows, n_columns, d_out, ws))) return rc;
+            if ((rc = acorr_device(h, d_in, n_rows, n_columns, d_out, z, tmp))) return rc;
         } else {  // a block of columns: gather it into a dense [n_rows][g] matrix, scatter the result back
             CU(cudaMemcpy2DAsync(c_in, (size_t)g * sizeof(double), d_in + c0, (size_t)n_columns * sizeof(double),
                                  (size_t)g * sizeof(double), n_rows, cudaMemcpyDeviceToDevice, st));
-            if ((rc = acorr_device(h, c_in, n_rows, g, c_out, ws))) return rc;
+            if ((rc = acorr_device(h, c_in, n_rows, g, c_out, z, tmp))) return rc;
             CU(cudaMemcpy2DAsync(d_out + c0, (size_t)n_columns * sizeof(double), c_out, (size_t)g * sizeof(double),
                                  (size_t)g * sizeof(double), n_rows, cudaMemcpyDeviceToDevice, st));
         }
@@ -390,15 +386,14 @@ int repet_beatspectrum_f64(repet_handle* h, const double* spectrogram, int n_fre
     const int L = next_pow2(2LL * n_times);
     const int chunk = (int)std::max<size_t>(1, std::min<size_t>((size_t)n_frequencies, ((size_t)2 << 30) / ((size_t)L * sizeof(double2))));
     const size_t n = (size_t)n_frequencies * n_times;
-    const size_t need = align_up(n * sizeof(double)) + 2 * align_up((size_t)chunk * L * sizeof(double2)) +
-                        align_up((size_t)n_times * sizeof(double)) + 1024;
-    int rc = repet::ensure_arena(h, need);
+    double *d_v, *d_beat; double2 *z, *tmp;
+    int rc = carve_arena(h, [&](Bump& b) {
+        d_v = b.take<double>(n);
+        z = b.take<double2>((size_t)chunk * L);
+        tmp = b.take<double2>((size_t)chunk * L);
+        d_beat = b.take<double>(n_times);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    double* d_v = bump.take<double>(n);
-    double2* z = bump.take<double2>((size_t)chunk * L);
-    double2* tmp = bump.take<double2>((size_t)chunk * L);
-    double* d_beat = bump.take<double>(n_times);
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(d_v, spectrogram, n * sizeof(double), cudaMemcpyHostToDevice, st));
     CU(cudaMemsetAsync(d_beat, 0, (size_t)n_times * sizeof(double), st));

@@ -31,13 +31,13 @@ int hlp_stft(repet_handle* h, const float* signal, int n_channels, int64_t n_sam
     if (n_frames_out) *n_frames_out = T;
     const size_t n = (size_t)n_samples * n_channels;
     const size_t x_elems = (size_t)T * n_channels * XPITCH;
-    const size_t need = align_up(n * sizeof(float)) + align_up(x_elems * sizeof(float2)) + align_up((size_t)T * PPITCH * sizeof(float));
-    int rc = ensure_arena(h, need);
+    float *in, *P; float2* X;
+    int rc = carve_arena(h, [&](Bump& b) {
+        in = b.take<float>(n);
+        X = b.take<float2>(x_elems);
+        P = b.take<float>((size_t)T * PPITCH);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float* in = bump.take<float>(n);
-    float2* X = bump.take<float2>(x_elems);
-    float* P = bump.take<float>((size_t)T * PPITCH);
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(in, signal, n * sizeof(float), cudaMemcpyHostToDevice, st));
     Geom g{1, 1, 0, 0, n_samples, 0, (int)n_samples, T};
@@ -59,12 +59,12 @@ int hlp_istft(repet_handle* h, const float* spectrum, int n_channels, int n_fram
     CU(cudaSetDevice(h->device));
     const long long S = (long long)(n_frames - 1) * HOP;
     const size_t x_elems = (size_t)n_frames * n_channels * XPITCH;
-    const size_t need = align_up(x_elems * sizeof(float2)) + align_up((size_t)S * n_channels * sizeof(float));
-    int rc = ensure_arena(h, need);
+    float2* X; float* out;
+    int rc = carve_arena(h, [&](Bump& b) {
+        X = b.take<float2>(x_elems);
+        out = b.take<float>((size_t)S * n_channels);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float2* X = bump.take<float2>(x_elems);
-    float* out = bump.take<float>((size_t)S * n_channels);
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(X, spectrum, x_elems * sizeof(float2), cudaMemcpyHostToDevice, st));
     Geom g{1, 1, 0, 0, S, 0, (int)S, n_frames};
@@ -86,15 +86,14 @@ int hlp_beat_common(repet_handle* h, const float* spectrogram, int n_frames, int
         return fail(h, REPET_E_UNSUPPORTED, "n_frames + max lag exceeds the 2048-point beat transform");
     CU(cudaSetDevice(h->device));
     const int n_parts = 17, f_per_part = 64;
-    const size_t need = align_up((size_t)n_frames * PPITCH * sizeof(float)) + align_up((size_t)n_parts * BEAT_L * sizeof(float)) +
-                        align_up((size_t)BEAT_L * sizeof(double)) + 512;
-    int rc = ensure_arena(h, need);
+    float *P, *psd; double* b; int32_t* per;
+    int rc = carve_arena(h, [&](Bump& w) {
+        P = w.take<float>((size_t)n_frames * PPITCH);
+        psd = w.take<float>((size_t)n_parts * BEAT_L);
+        b = w.take<double>(BEAT_L);
+        per = w.take<int32_t>(1);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float* P = bump.take<float>((size_t)n_frames * PPITCH);
-    float* psd = bump.take<float>((size_t)n_parts * BEAT_L);
-    double* b = bump.take<double>(BEAT_L);
-    int32_t* per = bump.take<int32_t>(1);
     cudaStream_t st = h->stream;
     CU(cudaMemsetAsync(P, 0, (size_t)n_frames * PPITCH * sizeof(float), st));
     CU(cudaMemcpy2DAsync(P, PPITCH * sizeof(float), spectrogram, n_rows * sizeof(float), n_rows * sizeof(float),
@@ -126,15 +125,14 @@ int hlp_mask(repet_handle* h, const float* magnitude, int n_frames, int period, 
     CU(cudaSetDevice(h->device));
     const int T = n_frames;
     const size_t x_elems = (size_t)T * XPITCH;
-    const size_t need = align_up(x_elems * sizeof(float2)) + align_up((size_t)period * PPITCH * sizeof(float)) +
-                        align_up((size_t)T * PPITCH * sizeof(float)) + 512;
-    int rc = ensure_arena(h, need);
+    float2* X; float *model, *M; int32_t* per;
+    int rc = carve_arena(h, [&](Bump& b) {
+        X = b.take<float2>(x_elems);
+        model = b.take<float>((size_t)period * PPITCH);
+        M = b.take<float>((size_t)T * PPITCH);
+        per = b.take<int32_t>(1);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float2* X = bump.take<float2>(x_elems);
-    float* model = bump.take<float>((size_t)period * PPITCH);
-    float* M = bump.take<float>((size_t)T * PPITCH);
-    int32_t* per = bump.take<int32_t>(1);
     std::vector<float2> host;
     pack_magnitudes(magnitude, T, host);
     cudaStream_t st = h->stream;
@@ -158,15 +156,14 @@ int hlp_adaptivemask(repet_handle* h, const float* magnitude, int n_frames, cons
     CU(cudaSetDevice(h->device));
     const int T = n_frames;
     const size_t x_elems = (size_t)T * XPITCH;
-    const size_t need = align_up(x_elems * sizeof(float2)) + 2 * align_up((size_t)T * PPITCH * sizeof(float)) +
-                        align_up((size_t)T * sizeof(int32_t)) + 512;
-    int rc = ensure_arena(h, need);
+    float2* X; float *model, *M; int32_t* per;
+    int rc = carve_arena(h, [&](Bump& b) {
+        X = b.take<float2>(x_elems);
+        model = b.take<float>((size_t)T * PPITCH);
+        M = b.take<float>((size_t)T * PPITCH);
+        per = b.take<int32_t>(T);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float2* X = bump.take<float2>(x_elems);
-    float* model = bump.take<float>((size_t)T * PPITCH);
-    float* M = bump.take<float>((size_t)T * PPITCH);
-    int32_t* per = bump.take<int32_t>(T);
     std::vector<float2> host;
     pack_magnitudes(magnitude, T, host);
     cudaStream_t st = h->stream;
@@ -193,15 +190,13 @@ int hlp_beatspectrogram(repet_handle* h, const float* spectrogram, int n_frames,
     const int n_seg = (n_frames + segment_step - 1) / segment_step;
     if (n_segments_out) *n_segments_out = n_seg;
     const int n_parts = 9, f_per_part = 120;
-    const size_t need = align_up((size_t)n_frames * PPITCH * sizeof(float)) +
-                        align_up((size_t)n_seg * n_parts * BEAT_L * sizeof(float)) +
-                        align_up((size_t)n_seg * segment_length * sizeof(double)) + 512;
-    int rc = ensure_arena(h, need);
+    float *P, *psd; double* b;
+    int rc = carve_arena(h, [&](Bump& w) {
+        P = w.take<float>((size_t)n_frames * PPITCH);
+        psd = w.take<float>((size_t)n_seg * n_parts * BEAT_L);
+        b = w.take<double>((size_t)n_seg * segment_length);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float* P = bump.take<float>((size_t)n_frames * PPITCH);
-    float* psd = bump.take<float>((size_t)n_seg * n_parts * BEAT_L);
-    double* b = bump.take<double>((size_t)n_seg * segment_length);
     cudaStream_t st = h->stream;
     CU(cudaMemsetAsync(P, 0, (size_t)n_frames * PPITCH * sizeof(float), st));
     CU(cudaMemcpy2DAsync(P, PPITCH * sizeof(float), spectrogram, n_rows * sizeof(float), n_rows * sizeof(float), n_frames,
@@ -223,15 +218,14 @@ int hlp_selfsimilarity(repet_handle* h, const float* magnitude, int n_frames, in
         return fail(h, REPET_E_INVALID_ARG, "bad buffer or size (n_rows <= window_length / 2 + 1)");
     CU(cudaSetDevice(h->device));
     const int T = n_frames;
-    const size_t need = align_up((size_t)T * PPITCH * sizeof(float)) + 2 * align_up((size_t)T * KPAD * sizeof(float)) +
-                        align_up((size_t)T * T * sizeof(float)) + 512;
-    int rc = ensure_arena(h, need);
+    float *V, *An32, *An32lo, *S;
+    int rc = carve_arena(h, [&](Bump& b) {
+        V = b.take<float>((size_t)T * PPITCH);
+        An32 = b.take<float>((size_t)T * KPAD);
+        An32lo = b.take<float>((size_t)T * KPAD);
+        S = b.take<float>((size_t)T * T);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float* V = bump.take<float>((size_t)T * PPITCH);
-    float* An32 = bump.take<float>((size_t)T * KPAD);
-    float* An32lo = bump.take<float>((size_t)T * KPAD);
-    float* S = bump.take<float>((size_t)T * T);
     cudaStream_t st = h->stream;
     CU(cudaMemsetAsync(V, 0, (size_t)T * PPITCH * sizeof(float), st));
     CU(cudaMemcpy2DAsync(V, PPITCH * sizeof(float), magnitude, n_rows * sizeof(float), n_rows * sizeof(float), T,
@@ -260,11 +254,12 @@ int hlp_periods(repet_handle* h, const double* beat, int n_lags, int n_columns, 
         return fail(h, REPET_E_TOO_SHORT, "attempt to get argmax of an empty sequence");
     CU(cudaSetDevice(h->device));
     const size_t n = (size_t)n_lags * n_columns;
-    int rc = ensure_arena(h, align_up(n * sizeof(double)) + align_up((size_t)n_columns * sizeof(int32_t)));
+    double* b; int32_t* per;
+    int rc = carve_arena(h, [&](Bump& w) {
+        b = w.take<double>(n);
+        per = w.take<int32_t>(n_columns);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    double* b = bump.take<double>(n);
-    int32_t* per = bump.take<int32_t>(n_columns);
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(b, beat, n * sizeof(double), cudaMemcpyHostToDevice, st));
     launch_argmax_columns(st, b, n_lags, n_columns, period_lo, lag_hi, per);
@@ -290,14 +285,13 @@ int hlp_similarity(repet_handle* h, const float* magnitude1, int n_frames1, cons
         return fail(h, REPET_E_INVALID_ARG, "bad buffer or size (n_rows <= window_length / 2 + 1)");
     CU(cudaSetDevice(h->device));
     const size_t n1 = n_frames1, n2 = n_frames2;
-    const size_t need = align_up((n1 + n2) * PPITCH * sizeof(float)) + align_up((n1 + n2) * APITCH64 * sizeof(double)) +
-                        align_up(n1 * n2 * sizeof(double)) + 1024;
-    int rc = ensure_arena(h, need);
+    float* V; double *An, *out;
+    int rc = carve_arena(h, [&](Bump& b) {
+        V = b.take<float>((n1 + n2) * PPITCH);
+        An = b.take<double>((n1 + n2) * APITCH64);
+        out = b.take<double>(n1 * n2);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float* V = bump.take<float>((n1 + n2) * PPITCH);
-    double* An = bump.take<double>((n1 + n2) * APITCH64);
-    double* out = bump.take<double>(n1 * n2);
     cudaStream_t st = h->stream;
     if ((rc = upload_rows(h, magnitude1, n_frames1, n_rows, V))) return rc;
     if ((rc = upload_rows(h, magnitude2, n_frames2, n_rows, V + n1 * PPITCH))) return rc;
@@ -317,15 +311,14 @@ int hlp_localmaxima(repet_handle* h, const double* data, int n, int n_columns, d
         return fail(h, REPET_E_INVALID_ARG, "bad buffer or size");
     CU(cudaSetDevice(h->device));
     const size_t total = (size_t)n * n_columns, lists = (size_t)n_columns * number_values;
-    const size_t need = align_up(total * sizeof(double)) + align_up(lists * sizeof(int32_t)) +
-                        align_up((size_t)n_columns * sizeof(int32_t)) + align_up(lists * sizeof(double)) + 1024;
-    int rc = ensure_arena(h, need);
+    double *d, *val; int32_t *idx, *cnt;
+    int rc = carve_arena(h, [&](Bump& b) {
+        d = b.take<double>(total);
+        idx = b.take<int32_t>(lists);
+        cnt = b.take<int32_t>(n_columns);
+        val = b.take<double>(lists);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    double* d = bump.take<double>(total);
-    int32_t* idx = bump.take<int32_t>(lists);
-    int32_t* cnt = bump.take<int32_t>(n_columns);
-    double* val = bump.take<double>(lists);
     cudaStream_t st = h->stream;
     CU(cudaMemcpyAsync(d, data, total * sizeof(double), cudaMemcpyHostToDevice, st));
     if (launch_localmaxima64(st, d, n, n_columns, minimum_value, minimum_distance, number_values, idx, cnt, val))
@@ -347,17 +340,16 @@ int hlp_simmask(repet_handle* h, const float* magnitude, int n_frames, const int
     CU(cudaSetDevice(h->device));
     const int T = n_frames;
     const size_t x_elems = (size_t)T * XPITCH;
-    const size_t need = align_up(x_elems * sizeof(float2)) + 3 * align_up((size_t)T * PPITCH * sizeof(float)) +
-                        align_up((size_t)T * number * sizeof(int32_t)) + align_up((size_t)T * sizeof(int32_t)) + 1024;
-    int rc = ensure_arena(h, need);
+    float2* X; float *model, *M, *Vsq; int32_t *idx, *cnt;
+    int rc = carve_arena(h, [&](Bump& b) {
+        X = b.take<float2>(x_elems);
+        model = b.take<float>((size_t)T * PPITCH);
+        M = b.take<float>((size_t)T * PPITCH);
+        Vsq = b.take<float>((size_t)T * PPITCH);
+        idx = b.take<int32_t>((size_t)T * number);
+        cnt = b.take<int32_t>(T);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float2* X = bump.take<float2>(x_elems);
-    float* model = bump.take<float>((size_t)T * PPITCH);
-    float* M = bump.take<float>((size_t)T * PPITCH);
-    float* Vsq = bump.take<float>((size_t)T * PPITCH);
-    int32_t* idx = bump.take<int32_t>((size_t)T * number);
-    int32_t* cnt = bump.take<int32_t>(T);
     std::vector<float2> host;
     pack_magnitudes(magnitude, T, host);
     cudaStream_t st = h->stream;
@@ -383,14 +375,13 @@ int hlp_acorr(repet_handle* h, const float* data, int n_rows, int n_columns, dou
     CU(cudaSetDevice(h->device));
     // every column becomes one beat item whose only non-zero frequency row is that column
     const int chunk = std::max(1, std::min(n_columns, (int)(((size_t)512 << 20) / ((size_t)n_rows * PPITCH * sizeof(float)))));
-    const size_t need = align_up((size_t)chunk * n_rows * PPITCH * sizeof(float)) + align_up((size_t)chunk * BEAT_L * sizeof(float)) +
-                        align_up((size_t)chunk * n_rows * sizeof(double)) + 1024;
-    int rc = ensure_arena(h, need);
+    float *P, *psd; double* b;
+    int rc = carve_arena(h, [&](Bump& w) {
+        P = w.take<float>((size_t)chunk * n_rows * PPITCH);
+        psd = w.take<float>((size_t)chunk * BEAT_L);
+        b = w.take<double>((size_t)chunk * n_rows);
+    });
     if (rc) return rc;
-    Bump bump(h->arena);
-    float* P = bump.take<float>((size_t)chunk * n_rows * PPITCH);
-    float* psd = bump.take<float>((size_t)chunk * BEAT_L);
-    double* b = bump.take<double>((size_t)chunk * n_rows);
     cudaStream_t st = h->stream;
     std::vector<double> host((size_t)chunk * n_rows);
     for (int c0 = 0; c0 < n_columns; c0 += chunk) {

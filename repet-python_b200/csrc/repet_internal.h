@@ -98,16 +98,22 @@ inline int fail(repet_handle* h, int code, const std::string& msg) {
 
 inline size_t align_up(size_t v, size_t a = 256) { return (v + a - 1) / a * a; }
 
+// Lays buffers out one after the other, each 256-byte aligned.  A layout is written once, as a sequence of takes,
+// and run twice: on Bump(nullptr), where take returns nullptr and only advances `off`, to measure it, and on the
+// memory it was measured for, to carve it.  `cap` is the size of that memory: a runner that carves from a
+// workspace it was handed checks `fits()` before it launches anything.
 struct Bump {
     unsigned char* base;
+    size_t cap;
     size_t off = 0;
-    explicit Bump(unsigned char* b) : base(b) {}
+    explicit Bump(unsigned char* b, size_t capacity = SIZE_MAX) : base(b), cap(capacity) {}
     template <typename T>
     T* take(size_t count) {
-        T* p = reinterpret_cast<T*>(base + off);
+        T* p = base ? reinterpret_cast<T*>(base + off) : nullptr;
         off = align_up(off + count * sizeof(T));
         return p;
     }
+    bool fits() const { return off <= cap; }
 };
 
 // Brackets the launches of one pipeline step with an event pair when profiling is on; always counts the
@@ -146,6 +152,18 @@ inline int ensure_arena(repet_handle* h, size_t bytes) {
     h->arena_bytes = 0;
     CU(cudaMalloc(&h->arena, bytes));
     h->arena_bytes = bytes;
+    return REPET_OK;
+}
+
+// Measures `layout` (a callable taking Bump&), grows the arena to its size and carves it from the arena.
+template <typename Layout>
+int carve_arena(repet_handle* h, Layout&& layout) {
+    Bump measure(nullptr);
+    layout(measure);
+    const int rc = ensure_arena(h, measure.off);
+    if (rc) return rc;
+    Bump bump(h->arena);
+    layout(bump);
     return REPET_OK;
 }
 

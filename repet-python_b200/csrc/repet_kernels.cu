@@ -481,8 +481,6 @@ void launch_periods(cudaStream_t st, const float* psd_part, const float* psd_par
 // clip) accumulated in float64 straight from P (the 1/F factor
 // is common), and the first maximum wins, as np.argmax does.  Unflagged clips cost one flag read.
 // ------------------------------------------------------------------------------------------
-constexpr int CERT_TSPLIT = 16;  // time chunks per candidate (partial sums are added in a fixed order)
-
 constexpr int CERT_GROUP = 32;   // beat items whose flags one CTA scans (one per lane of warp 0)
 
 __global__ void __launch_bounds__(256)

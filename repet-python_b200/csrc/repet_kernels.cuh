@@ -114,6 +114,9 @@ void launch_periods(cudaStream_t st, const float* psd_part, const float* psd_par
                     int beat_pitch, int* period, double* stats, int* cert, int L = BEAT_L);
 // near-tied period candidates re-decided in float64 (cert: [item][1 + CERT_MAX] ints written by k_periods)
 constexpr int CERT_MAX = 8;
+// k_period_certify splits each candidate's sum into CERT_TSPLIT time chunks (partial sums added in a fixed order):
+// cert_val is [item][CERT_MAX][CERT_TSPLIT] doubles
+constexpr int CERT_TSPLIT = 16;
 constexpr double CERT_REL = 1e-4;
 // n_items beat items = clips x n_seg segments of rows [t_first + seg*seg_step, ... + t_len) (original: 0, T, 0, 1)
 void launch_period_certify(cudaStream_t st, const float* P, int n_items, int T, int t_first, int t_len, int seg_step,

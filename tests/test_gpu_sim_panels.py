@@ -46,14 +46,14 @@ def _align(v):
 
 
 def _linear_bytes(T, nch, number, sm_count):
-    """Workspace of one `sim` track besides S, as make_plan (csrc/repet_drivers.cu) sums it at 44.1 kHz."""
+    """Workspace of one `sim` track besides S, as carve_sim (csrc/repet_drivers.cu) lays it out at 44.1 kHz."""
     xpitch, ppitch, kpad = 1024, 1032, 1056
     b = _align(T * nch * xpitch * 8) + _align(T * ppitch * 4) + _align(T * ppitch * 8) + _align(T * number * 4)
     b += _align(T * 4) + _align(nch * T * ppitch * 4)
     if number > 32:
         b += _align(nch * T * ppitch * 4)
-    b += 2 * _align(T * kpad * 4) + _align(T * 4) + _align((T * 12 + 255) // 256 * 256 * sm_count * 2)
-    return b + 2048
+    b += _align(4 * 4)  # k_topk's overflow counters
+    return b + 2 * _align(T * kpad * 4) + _align(T * 4) + _align((T * 12 + 255) // 256 * 256 * sm_count * 2)
 
 
 def _limit_for_rows(T, P, nch, sm_count, number=100):
