@@ -71,7 +71,10 @@ int repet_set_window(repet_handle* h, const double* window, int n);
  * device memory free when the handle first asks)).  A chunk never holds less than one clip, so one clip whose
  * workspace alone exceeds the cap still runs.  REPET-SIM honours the cap for long tracks too: when a track's
  * similarity matrix does not fit, it is formed and consumed in row panels as high as the cap leaves room for
- * (at least 128 rows), one track at a time.  Buffers an entry point stages its own input and output in come on top. */
+ * (at least 128 rows), one track at a time.  repet_general_f64's REPET-SIM honours the cap as well: its float64
+ * similarity matrix and selection scratch are formed in row panels (multiples of 64 rows, at least 64) when the whole
+ * matrix does not fit; its buffers that grow linearly with the track are not counted.  Buffers an entry point stages
+ * its own input and output in come on top. */
 int repet_set_workspace_limit(repet_handle* h, uint64_t bytes);
 /* Bytes of device workspace the handle holds now (it grows on demand and is kept for later calls). */
 uint64_t repet_workspace_bytes(repet_handle* h);
@@ -308,7 +311,12 @@ int repet_beatspectrum_f64(repet_handle* h, const double* spectrogram, int n_fre
  * points at 96 kHz, 8192 at 192 kHz, repet.py:130), any number of channels (repet.py:152-155), period ranges above
  * 1024 frames, segments longer than one beat transform.  float64 end to end on the device (integer decisions need no
  * certification), built for generality, not speed.  audio / background: (n_samples, n_channels) float64, HOST;
- * window: the analysis window (window_length doubles, HOST); ints_host as repet_ints_per_clip(method, p, n_samples). */
+ * window: the analysis window (window_length doubles, HOST); ints_host as repet_ints_per_clip(method, p, n_samples).
+ * REPET-SIM (method 3) forms the T x T float64 similarity matrix whole when it and the selection scratch fit the
+ * handle's workspace limit (repet_set_workspace_limit), else in row panels of the largest multiple of 64 rows that
+ * fits; the matrix is bitwise symmetric, so panels give the same lists and background bit for bit.  The buffers
+ * linear in T (spectra, magnitudes, staging: about 36 GB for one hour of 96 kHz mono) are outside the limit, and a
+ * clip needs T * window_length < 2e9 (about 2.9 h at 96 kHz) or the call returns REPET_E_UNSUPPORTED. */
 int repet_general_f64(repet_handle* h, int method, const double* audio, int64_t n_samples, int n_channels,
                       const repet_params* p, const double* window, double* background, int32_t* ints_host,
                       int64_t ints_capacity);

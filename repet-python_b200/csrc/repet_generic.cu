@@ -16,6 +16,7 @@ namespace {
 using repet::fail;
 using repet::Bump;
 using repet::carve_arena;
+using repet::default_ws_limit;
 
 __device__ __forceinline__ double2 zmul(double2 a, double2 b) {
     return make_double2(fma(a.x, b.x, -a.y * b.y), fma(a.x, b.y, a.y * b.x));
@@ -570,13 +571,15 @@ __global__ void k_gen_normalize(const double* __restrict__ Vm, long long T, int 
     const double norm = sqrt(s_red[0]);
     for (int f = threadIdx.x; f < F; f += blockDim.x) An[t * F + f] = Vm[t * F + f] / norm;
 }
-// S = An An^T, float64, 64 x 64 tiles; the k order is the same for (i, j) and (j, i): S is bitwise symmetric
+// Rows [r0, r0 + rows) of S = An An^T, float64, 64 x 64 tiles, into S row-major with pitch T (the whole matrix: r0 = 0,
+// rows = T).  Every element is one fma chain over ascending k from 0.0, whichever tile forms it, and fma(a, b, c) =
+// fma(b, a, c): S is bitwise symmetric, and a panel holds bit for bit the rows of the whole matrix.
 __global__ void __launch_bounds__(256)
-k_gen_gram(const double* __restrict__ An, long long T, int F, double* __restrict__ S) {
+k_gen_gram(const double* __restrict__ An, long long T, int F, long long r0, long long rows, double* __restrict__ S) {
     __shared__ double sa[16][65];
     __shared__ double sb[16][65];
     const int ti = threadIdx.x & 15, tj = threadIdx.x >> 4;
-    const long long i0 = (long long)blockIdx.y * 64, j0 = (long long)blockIdx.x * 64;
+    const long long i0 = (long long)blockIdx.x * 64, j0 = r0 + (long long)blockIdx.y * 64, j_end = r0 + rows;
     double acc[4][4] = {};
     for (int k0 = 0; k0 < F; k0 += 16) {
         for (int e = 0; e < 4; ++e) {
@@ -584,7 +587,7 @@ k_gen_gram(const double* __restrict__ An, long long T, int F, double* __restrict
             const int row = idx >> 4, kk = idx & 15;
             const long long ri = i0 + row, rj = j0 + row;
             sa[kk][row] = (ri < T && k0 + kk < F) ? An[ri * F + k0 + kk] : 0.0;
-            sb[kk][row] = (rj < T && k0 + kk < F) ? An[rj * F + k0 + kk] : 0.0;
+            sb[kk][row] = (rj < j_end && k0 + kk < F) ? An[rj * F + k0 + kk] : 0.0;
         }
         __syncthreads();
         for (int kk = 0; kk < 16; ++kk) {
@@ -599,7 +602,7 @@ k_gen_gram(const double* __restrict__ An, long long T, int F, double* __restrict
     for (int a = 0; a < 4; ++a)
         for (int b = 0; b < 4; ++b) {
             const long long i = i0 + ti + 16 * a, j = j0 + tj + 16 * b;
-            if (i < T && j < T) S[j * T + i] = acc[a][b];
+            if (i < T && j < j_end) S[(j - r0) * T + i] = acc[a][b];
         }
 }
 // _localmaxima of one vector held in shared memory (repet.py:1309-1343): v >= thr and strictly above every neighbour
@@ -624,7 +627,7 @@ __device__ void gen_localmaxima(const double* __restrict__ v, int n, double thr,
         const int i = kept[q];
         const double x = v[i];
         int rank = 0;
-        for (int r = 0; r < K; ++r) {
+        for (int r = 0; r < K && rank < number; ++r) {  // a candidate ranked `number` or below is out either way
             const int io = kept[r];
             rank += (v[io] > x) || (v[io] == x && io > i);
         }
@@ -640,20 +643,21 @@ __device__ void gen_localmaxima(const double* __restrict__ v, int n, double thr,
     if (threadIdx.x == 0) *cnt_out = min(K, number);
     __syncthreads();
 }
-// REPET-SIM: the similar-frame list of every column of S (repet.py:1370-1381).  Persistent CTAs walk the columns; a
-// column (= row of the symmetric S) is examined in chunks of GEN_IDX_CHUNK elements staged in shared memory with a
-// halo of d on both sides, so a track of any length fits; the survivors' indices go to a per-CTA global scratch list
-// and are ranked by value (ties: descending index) as _localmaxima does.
+// REPET-SIM: the similar-frame lists of columns r0 .. r0 + rows - 1 of S (repet.py:1370-1381), from the panel S that
+// holds rows [r0, r0 + rows) of the symmetric S with pitch T.  Persistent CTAs walk the columns; a column (= row of
+// S) is examined in chunks of GEN_IDX_CHUNK elements staged in shared memory with a halo of d on both sides, so a
+// track of any length fits; the survivors' indices go to a per-CTA global scratch list and are ranked by value (ties:
+// descending index) as _localmaxima does.  idx / cnt are indexed by absolute frame.
 constexpr int GEN_IDX_CHUNK = 4096;
 __global__ void __launch_bounds__(512)
-k_gen_indices(const double* __restrict__ S, int T, double thr, int d, int number, int* __restrict__ idx, int* __restrict__ cnt,
-              int* __restrict__ kept_scratch) {
+k_gen_indices(const double* __restrict__ S, int T, int r0, int rows, double thr, int d, int number, int* __restrict__ idx,
+              int* __restrict__ cnt, int* __restrict__ kept_scratch) {
     extern __shared__ __align__(16) unsigned char gsm[];
     double* v = reinterpret_cast<double*>(gsm);  // [GEN_IDX_CHUNK + 2 d]
     __shared__ int s_count;
     int* __restrict__ kept = kept_scratch + (size_t)blockIdx.x * T;
-    for (int c = blockIdx.x; c < T; c += gridDim.x) {
-        const double* __restrict__ row = S + (long long)c * T;
+    for (int c = r0 + blockIdx.x; c < r0 + rows; c += gridDim.x) {
+        const double* __restrict__ row = S + (long long)(c - r0) * T;
         __syncthreads();
         if (threadIdx.x == 0) s_count = 0;
         for (int g0 = 0; g0 < T; g0 += GEN_IDX_CHUNK) {
@@ -682,7 +686,7 @@ k_gen_indices(const double* __restrict__ S, int T, double thr, int d, int number
             const int i = kept[q];
             const double a = row[i];
             int rank = 0;
-            for (int r = 0; r < K; ++r) {
+            for (int r = 0; r < K && rank < number; ++r) {  // a candidate ranked `number` or below is out either way
                 const int io = kept[r];
                 const double b = row[io];
                 rank += (b > a) || (b == a && io > i);
@@ -986,18 +990,37 @@ int gen_run(repet_handle* h, int method, const double* d_audio, long long S, int
                                                                             p->similarity_threshold, p->similarity_distance,
                                                                             number, idx, cnt);
         } else {
-            double* Sm = pool.get<double>((size_t)T * T);
-            if (!pool.ok) return fail(h, REPET_E_OOM, "out of device memory for the similarity matrix");
-            dim3 grid((unsigned)((T + 63) / 64), (unsigned)((T + 63) / 64));
-            k_gen_gram<<<grid, 256, 0, st>>>(An, T, F, Sm);
             const size_t smem = (size_t)(GEN_IDX_CHUNK + 2 * (size_t)p->similarity_distance) * sizeof(double);
             if (smem > 200 * 1024) return fail(h, REPET_E_UNSUPPORTED, "similarity_distance too long for the general similar-frame selection");
             if (smem > 48 * 1024) CU(cudaFuncSetAttribute(k_gen_indices, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem));
-            const int n_ctas = (int)std::min<long long>(T, 2LL * h->sm_count);
-            int* kept_scratch = pool.get<int>((size_t)n_ctas * T);
-            if (!pool.ok) return fail(h, REPET_E_OOM, "out of device memory in the general path");
-            k_gen_indices<<<n_ctas, 512, smem, st>>>(Sm, (int)T, p->similarity_threshold, p->similarity_distance, number, idx, cnt,
-                                                     kept_scratch);
+            // S and k_gen_indices' per-CTA kept lists are the quadratic part of the call, and the workspace limit
+            // governs them: need(P) = P rows of S + one list of T ints per selection CTA.  The whole matrix when
+            // need(T) fits; otherwise panels of P rows, the largest multiple of the Gram tile (64) that fits, 64 at
+            // least.  S is bitwise symmetric, so a panel's rows are the columns whose lists it settles: panels give
+            // the whole matrix's lists exactly.  The linear buffers (X, tmp, V, Vm, An and the entry point's staging)
+            // are not counted against the limit.
+            const long long max_ctas = 2LL * h->sm_count;
+            auto need = [&](long long P) { return (size_t)P * T * sizeof(double) + (size_t)std::min(P, max_ctas) * T * sizeof(int); };
+            const size_t limit = default_ws_limit(h);
+            long long P = T;
+            if (need(T) > limit) {
+                P = std::min<long long>(T, (long long)(limit / ((size_t)T * sizeof(double)))) / 64 * 64;
+                while (P > 64 && need(P) > limit) P -= 64;
+                P = std::min(T, std::max(P, 64LL));
+            }
+            double* Sm = pool.get<double>((size_t)P * T);
+            int* kept_scratch = pool.get<int>((size_t)std::min(P, max_ctas) * T);
+            if (!pool.ok) return fail(h, REPET_E_OOM, "out of device memory for the similarity matrix");
+            for (long long r0 = 0; r0 < T; r0 += P) {
+                const long long rows = std::min(P, T - r0);
+                dim3 grid((unsigned)((T + 63) / 64), (unsigned)((rows + 63) / 64));
+                k_gen_gram<<<grid, 256, 0, st>>>(An, T, F, r0, rows, Sm);
+                k_gen_indices<<<(unsigned)std::min(rows, max_ctas), 512, smem, st>>>(Sm, (int)T, (int)r0, (int)rows,
+                                                                                    p->similarity_threshold,
+                                                                                    p->similarity_distance, number, idx,
+                                                                                    cnt, kept_scratch);
+                h->launches += 2;
+            }
             pool.release(kept_scratch);
             pool.release(Sm);
         }
