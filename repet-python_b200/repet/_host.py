@@ -335,6 +335,9 @@ def number_of_frames(number_samples, window_length, step_length):
 # drivers
 # ------------------------------------------------------------------------------------------
 FAST_WINDOWS = (512, 1024, 2048)  # window lengths of the register-blocked fp32 frame transforms
+METHODS = {"original": 0, "extended": 1, "adaptive": 2, "sim": 3, "simonline": 4}
+FORMATS = {"f32": 0, "pcm16": 1}  # REPET_FMT_F32_PLANAR, REPET_FMT_PCM16
+SPECTROGRAMS = ("audio_spectrogram", "background_spectrogram", "foreground_spectrogram")
 
 
 def needs_general_path(params, number_channels):
@@ -345,15 +348,95 @@ def needs_general_path(params, number_channels):
     return params.window_length not in FAST_WINDOWS or number_channels > 2
 
 
-def general_f64(method, audio_signal, sampling_frequency, tunables, handle=None):
-    """Any of the five drivers on the general float64 device path.  Returns (background float64 (S, C), ints int32)."""
-    number_samples, number_channels = np.shape(audio_signal)
+def _route(params, number_channels, fast, general):
+    """The one rule between the two device paths: `fast()`, unless the fast kernels are not compiled for the input
+    (needs_general_path) or refuse it (NotImplementedError, i.e. REPET_E_UNSUPPORTED: a period range above 1024
+    frames, ...); then `general()`.  Every other error propagates."""
+    if not needs_general_path(params, number_channels):
+        try:
+            return fast()
+        except NotImplementedError:
+            pass
+    return general()
+
+
+def _ints_per_clip(lib, method, params, number_samples):
+    return int(lib.repet_ints_per_clip(METHODS[method], ctypes.byref(params), number_samples))
+
+
+def _run_f64(method, audio_signal, params, window_function, handle=None, foreground=False, spectrograms=False):
+    """One clip of `method`, float64 (samples, channels) in and out, on the path _route picks.  `params` and
+    `window_function` come from derive_params (callers may set online_frame_base).  Returns a dict: background,
+    integers (the method's integer output), and on request foreground and the three display spectrograms
+    (SPECTROGRAMS, which need `foreground` too)."""
+    _, number_channels = np.shape(audio_signal)  # ValueError if not 2-D, as in the reference
     handle = handle or get_handle()
-    params, window_function = derive_params(sampling_frequency, tunables, method)
+    return _route(params, number_channels,
+                  lambda: _fast_f64(method, audio_signal, params, handle, foreground, spectrograms),
+                  lambda: _general_f64(method, audio_signal, params, window_function, handle, foreground, spectrograms))
+
+
+def _fast_f64(method, audio_signal, params, handle, foreground=False, spectrograms=False):
+    """The fast route of _run_f64 (repet_separate_f64) alone: raises NotImplementedError where the fast kernels
+    refuse the input.  The foreground and the spectrograms are formed on the device from the buffers already there."""
     audio = np.ascontiguousarray(audio_signal, dtype=np.float64)
-    window = np.ascontiguousarray(window_function, dtype=np.float64)
+    number_samples, number_channels = audio.shape
+    lib = handle.lib
+    handle.ensure_window(params.window_length)
+    capacity = _ints_per_clip(lib, method, params, number_samples)
+    background = np.empty_like(audio)
+    ints = np.zeros(max(1, capacity), dtype=np.int32)
+    fg = np.empty_like(audio) if foreground else None
+    spec = None
+    if spectrograms:
+        spec = np.empty((3, lib.repet_spectrogram_frames(ctypes.byref(params), number_samples),
+                         lib.repet_spectrogram_pitch(ctypes.byref(params))), dtype=np.float32)
+    handle.check(
+        lib.repet_separate_f64(
+            handle.h, METHODS[method], _ptr(audio), number_samples, number_channels, ctypes.byref(params),
+            _ptr(background), _ptr(fg), _ptr(spec), _ptr(ints), len(ints),
+        )
+    )
+    result = {"background": background}
+    if foreground:
+        result["foreground"] = fg
+    result["integers"] = ints[:capacity]
+    if spectrograms:
+        number_frequencies = params.window_length // 2 + 1
+        for i, name in enumerate(SPECTROGRAMS):
+            result[name] = spec[i, :, :number_frequencies].T.astype(np.float64)
+    return result
+
+
+def _single_f64_fast(entry, driver, audio_signal, sampling_frequency, tunables, handle, ints_capacity):
+    """The fast kernels alone through a per-driver entry point `entry` (repet_<driver>_f64, kept public for C
+    integrators): no routing, so a refusal raises NotImplementedError.  For tests that need the fast kernels' own
+    answer on that entry point; `ints_capacity(params, number_samples)` sizes the integer output."""
+    number_samples, number_channels = np.shape(audio_signal)
+    params, _ = derive_params(sampling_frequency, tunables, driver)
+    handle.ensure_window(params.window_length)
+    audio = np.ascontiguousarray(audio_signal, dtype=np.float64)
     background = np.empty((number_samples, number_channels), dtype=np.float64)
-    capacity = int(handle.lib.repet_ints_per_clip(METHODS[method], ctypes.byref(params), number_samples))
+    capacity = ints_capacity(params, number_samples)
+    ints = np.zeros(max(1, capacity), dtype=np.int32)
+    handle.check(
+        getattr(handle.lib, entry)(
+            handle.h, _ptr(audio), number_samples, number_channels, ctypes.byref(params), _ptr(background), _ptr(ints),
+            len(ints),
+        )
+    )
+    return background, ints[:capacity]
+
+
+def _general_f64(method, audio_signal, params, window_function, handle, foreground=False, spectrograms=False):
+    """The general route of _run_f64 (repet_general_f64).  The foreground and the spectrograms are formed on the
+    host from its outputs (foreground = audio - background, README.md:68; spectrograms by the general _stft,
+    README.md:79-81)."""
+    audio = np.ascontiguousarray(audio_signal, dtype=np.float64)
+    number_samples, number_channels = audio.shape
+    window = np.ascontiguousarray(window_function, dtype=np.float64)
+    capacity = _ints_per_clip(handle.lib, method, params, number_samples)
+    background = np.empty_like(audio)
     ints = np.zeros(max(1, capacity), dtype=np.int32)
     handle.check(
         handle.lib.repet_general_f64(
@@ -361,67 +444,97 @@ def general_f64(method, audio_signal, sampling_frequency, tunables, handle=None)
             _ptr(background), _ptr(ints), len(ints),
         )
     )
-    return background, ints[:capacity]
+    result = {"background": background}
+    if foreground:
+        result["foreground"] = audio - background
+    result["integers"] = ints[:capacity]
+    if spectrograms:
+        half = params.window_length // 2 + 1
+        for name, signal in zip(SPECTROGRAMS, (audio, background, result["foreground"])):
+            result[name] = np.abs(stft_general(np.mean(signal, axis=1), window_function, params.step_length,
+                                               handle=handle)[0:half, :])
+    return result
+
+
+def _run_batch(method, audio, params, window_function, handle=None, in_format="f32", out_format="f32", out=None,
+               devices=None):
+    """A batch of equally long clips of `method` in host memory, on the path _route picks: the fast kernels
+    (repet_separate_batch, clip-sharded over `devices` when given; a refusal of any shard sends the whole batch to
+    the general path), or clip by clip the general float64 path on the caller's handle.  Returns (background in
+    `out_format`, integers (clips, max(1, per clip)) int32)."""
+    in_code, out_code = FORMATS[in_format], FORMATS[out_format]
+    audio = np.ascontiguousarray(audio, dtype=np.int16 if in_code else np.float32)
+    if audio.ndim != 3:
+        raise ValueError("audio must have shape (clips, channels, samples) [f32] or (clips, samples, channels) [pcm16]")
+    if in_code:
+        number_clips, number_samples, number_channels = audio.shape
+    else:
+        number_clips, number_channels, number_samples = audio.shape
+    out_shape = (number_clips, number_samples, number_channels) if out_code else (number_clips, number_channels, number_samples)
+    out_dtype = np.int16 if out_code else np.float32
+    if out is None:
+        out = np.empty(out_shape, dtype=out_dtype)
+    elif out.shape != out_shape or out.dtype != out_dtype or not out.flags.c_contiguous:
+        raise ValueError("out must be a C-contiguous %s array of shape %s" % (np.dtype(out_dtype).name, out_shape))
+    if devices is not None:
+        devices = [int(d) for d in devices]
+    per_clip = _ints_per_clip(load_library(), method, params, number_samples)
+    ints = np.zeros((number_clips, max(1, per_clip)), dtype=np.int32)
+
+    def run(h, first, stop):
+        if stop <= first:
+            return
+        h.ensure_window(params.window_length)
+        h.check(h.lib.repet_separate_batch(
+            h.h, METHODS[method], _ptr(audio[first:stop]), in_code, stop - first, number_channels, number_samples,
+            ctypes.byref(params), _ptr(out[first:stop]), out_code, _ptr(ints[first:stop])))
+
+    def fast():
+        if devices is None:
+            run(handle or get_handle(), 0, number_clips)
+        else:
+            shards = shard_bounds(number_clips, len(devices))
+            _run_shards([(lambda h, lo=lo, hi=hi: run(h, lo, hi)) for lo, hi in shards], devices)
+        return out, ints
+
+    def general():
+        h = handle or get_handle()
+        for i, clip in enumerate(audio):
+            x = clip / 32768.0 if in_code else clip.T  # repet.py:929
+            result = _general_f64(method, x, params, window_function, h)
+            y = result["background"]
+            if out_code:
+                out[i] = np.clip(np.rint(y.astype(np.float32) * np.float32(32768.0)), -32768, 32767).astype(np.int16)
+            else:
+                out[i] = y.T
+            ints[i, : len(result["integers"])] = result["integers"]
+        return out, ints
+
+    return _route(params, number_channels, fast, general)
+
+
+def general_f64(method, audio_signal, sampling_frequency, tunables, handle=None):
+    """Any of the five drivers on the general float64 device path.  Returns (background float64 (S, C), ints int32)."""
+    params, window_function = derive_params(sampling_frequency, tunables, method)
+    result = _general_f64(method, audio_signal, params, window_function, handle or get_handle())
+    return result["background"], result["integers"]
 
 
 def original_f64(audio_signal, sampling_frequency, tunables, handle=None, return_period=False):
     """repet.original with the reference's calling convention (repet.py:67-202)."""
-    number_samples, number_channels = np.shape(audio_signal)  # repet.py:125 (ValueError if not 2-D)
-    handle = handle or get_handle()
     params, window_function = derive_params(sampling_frequency, tunables)
-    if needs_general_path(params, number_channels):
-        background, ints = general_f64("original", audio_signal, sampling_frequency, tunables, handle=handle)
-        return (background, int(ints[0])) if return_period else background
-    try:
-        return _original_f64_fast(audio_signal, sampling_frequency, tunables, handle, return_period)
-    except NotImplementedError:  # e.g. a period range above 1024 frames: the general path has no such limit
-        background, ints = general_f64("original", audio_signal, sampling_frequency, tunables, handle=handle)
-        return (background, int(ints[0])) if return_period else background
-
-
-def _original_f64_fast(audio_signal, sampling_frequency, tunables, handle, return_period):
-    number_samples, number_channels = np.shape(audio_signal)
-    params, window_function = derive_params(sampling_frequency, tunables)
-    handle.ensure_window(params.window_length)
-    audio = np.ascontiguousarray(audio_signal, dtype=np.float64)
-    background = np.empty((number_samples, number_channels), dtype=np.float64)
-    period = np.zeros(1, dtype=np.int32)
-    handle.check(
-        handle.lib.repet_original_f64(
-            handle.h, _ptr(audio), number_samples, number_channels, ctypes.byref(params), _ptr(background), _ptr(period)
-        )
-    )
+    result = _run_f64("original", audio_signal, params, window_function, handle)
     if return_period:
-        return background, int(period[0])
-    return background
+        return result["background"], int(result["integers"][0])
+    return result["background"]
 
 
 def original_batch(audio, sampling_frequency, tunables, handle=None, out=None):
     """`original` over a batch of clips: audio (B, C, S) float32 planar, host memory.
     Returns (background (B, C, S) float32, periods (B,) int32)."""
-    handle = handle or get_handle()
-    audio = np.ascontiguousarray(audio, dtype=np.float32)
-    if audio.ndim != 3:
-        raise ValueError("audio must have shape (clips, channels, samples)")
-    number_clips, number_channels, number_samples = audio.shape
-    params, _ = derive_params(sampling_frequency, tunables)
-    if needs_general_path(params, number_channels):
-        background, ints = _separate_batch_general("original", audio, 0, 0, sampling_frequency, tunables, handle, out)
-        return background, ints[:, 0]
-    handle.ensure_window(params.window_length)
-    background = out if out is not None else np.empty_like(audio)
-    periods = np.zeros(number_clips, dtype=np.int32)
-    try:
-        handle.check(
-            handle.lib.repet_original_batch(
-                handle.h, _ptr(audio), number_clips, number_channels, number_samples, ctypes.byref(params),
-                _ptr(background), _ptr(periods),
-            )
-        )
-    except NotImplementedError:  # e.g. a period range above 1024 frames: the general path has no such limit
-        background, ints = _separate_batch_general("original", audio, 0, 0, sampling_frequency, tunables, handle, out)
-        return background, ints[:, 0]
-    return background, periods
+    params, window_function = derive_params(sampling_frequency, tunables)
+    background, ints = _run_batch("original", audio, params, window_function, handle, out=out)
+    return background, ints[:, 0]
 
 
 def original_batch_device(audio_ptr, background_ptr, number_clips, number_channels, number_samples,
@@ -603,39 +716,6 @@ def mask(audio_spectrogram, repeating_period, handle=None):
     return out.T.astype(np.float64)
 
 
-def _single_f64(entry, driver, audio_signal, sampling_frequency, tunables, handle, ints_capacity):
-    number_samples, number_channels = np.shape(audio_signal)  # ValueError if not 2-D, as in the reference
-    handle = handle or get_handle()
-    params, _ = derive_params(sampling_frequency, tunables, driver)
-    if needs_general_path(params, number_channels):
-        ints_capacity(params, number_samples)  # (lets the caller record the frame count)
-        return general_f64(driver, audio_signal, sampling_frequency, tunables, handle=handle)
-    try:
-        return _single_f64_fast(entry, driver, audio_signal, sampling_frequency, tunables, handle, ints_capacity)
-    except NotImplementedError:
-        return general_f64(driver, audio_signal, sampling_frequency, tunables, handle=handle)
-
-
-def _single_f64_fast(entry, driver, audio_signal, sampling_frequency, tunables, handle, ints_capacity):
-    number_samples, number_channels = np.shape(audio_signal)
-    params, _ = derive_params(sampling_frequency, tunables, driver)
-    handle.ensure_window(params.window_length)
-    audio = np.ascontiguousarray(audio_signal, dtype=np.float64)
-    background = np.empty((number_samples, number_channels), dtype=np.float64)
-    capacity = ints_capacity(params, number_samples)
-    ints = np.zeros(max(1, capacity), dtype=np.int32)
-    handle.check(
-        getattr(handle.lib, entry)(
-            handle.h, _ptr(audio), number_samples, number_channels, ctypes.byref(params), _ptr(background), _ptr(ints),
-            len(ints),
-        )
-    )
-    return background, ints[:capacity]
-
-
-METHODS = {"original": 0, "extended": 1, "adaptive": 2, "sim": 3, "simonline": 4}
-
-
 def separate_f64(method, audio_signal, sampling_frequency, tunables, handle=None, spectrograms=True):
     """One call for the reference's documented usage (README.md:64-81): background by `method`,
     foreground = audio - background, and the display spectrograms abs(_stft(mean(x, axis=1)))[0:F] of
@@ -645,54 +725,8 @@ def separate_f64(method, audio_signal, sampling_frequency, tunables, handle=None
     float64 (when `spectrograms`); integers = the method's integer output (period(s) or packed lists)."""
     if method not in METHODS:
         raise ValueError("method must be one of %s" % sorted(METHODS))
-    number_samples, number_channels = np.shape(audio_signal)
-    handle = handle or get_handle()
-    lib = handle.lib
     params, window_function = derive_params(sampling_frequency, tunables, method)
-    if needs_general_path(params, number_channels):
-        # general float64 path: the by-products are formed from its outputs (foreground = audio - background,
-        # README.md:68; spectrograms by the general _stft, README.md:79-81)
-        audio = np.asarray(audio_signal, dtype=np.float64)
-        background, ints = general_f64(method, audio, sampling_frequency, tunables, handle=handle)
-        result = {"background": background, "foreground": audio - background, "integers": ints}
-        if spectrograms:
-            half = params.window_length // 2 + 1
-            for name, signal in (("audio_spectrogram", audio), ("background_spectrogram", background),
-                                 ("foreground_spectrogram", result["foreground"])):
-                result[name] = np.abs(stft_general(np.mean(signal, axis=1), window_function, params.step_length,
-                                                   handle=handle)[0:half, :])
-        return result
-    handle.ensure_window(params.window_length)
-    audio = np.ascontiguousarray(audio_signal, dtype=np.float64)
-    background = np.empty((number_samples, number_channels), dtype=np.float64)
-    foreground = np.empty((number_samples, number_channels), dtype=np.float64)
-    number_frames = lib.repet_spectrogram_frames(ctypes.byref(params), number_samples)
-    number = int(tunables["similarity_number"])
-    if method == "original":
-        capacity = 1
-    elif method == "extended":
-        capacity = max(1, lib.repet_extended_segments(ctypes.byref(params), number_samples))
-    elif method == "adaptive":
-        capacity = number_frames
-    elif method == "sim":
-        capacity = number_frames * (number + 1)
-    else:
-        capacity = max(0, lib.repet_simonline_frames(ctypes.byref(params), number_samples)) * (number + 1)
-    ints = np.zeros(max(1, capacity), dtype=np.int32)
-    pitch = lib.repet_spectrogram_pitch(ctypes.byref(params))
-    spec = np.empty((3, number_frames, pitch), dtype=np.float32) if spectrograms else None
-    handle.check(
-        lib.repet_separate_f64(
-            handle.h, METHODS[method], _ptr(audio), number_samples, number_channels, ctypes.byref(params),
-            _ptr(background), _ptr(foreground), _ptr(spec), _ptr(ints), len(ints),
-        )
-    )
-    result = {"background": background, "foreground": foreground, "integers": ints[:capacity]}
-    if spectrograms:
-        number_frequencies = params.window_length // 2 + 1
-        for i, name in enumerate(("audio_spectrogram", "background_spectrogram", "foreground_spectrogram")):
-            result[name] = spec[i, :, :number_frequencies].T.astype(np.float64)
-    return result
+    return _run_f64(method, audio_signal, params, window_function, handle, foreground=True, spectrograms=spectrograms)
 
 
 def spectrogram_batch_device(audio_ptr, spectrogram_ptr, number_clips, number_channels, number_samples,
@@ -721,66 +755,25 @@ def foreground_device(audio_ptr, background_ptr, foreground_ptr, number_elements
 
 def extended_f64(audio_signal, sampling_frequency, tunables, handle=None, return_periods=False):
     """repet.extended with the reference's calling convention (repet.py:205-419)."""
-    lib = load_library()
-    background, periods = _single_f64(
-        "repet_extended_f64", "extended", audio_signal, sampling_frequency, tunables, handle,
-        lambda params, number_samples: lib.repet_extended_segments(ctypes.byref(params), number_samples),
-    )
-    return (background, periods) if return_periods else background
+    params, window_function = derive_params(sampling_frequency, tunables, "extended")
+    result = _run_f64("extended", audio_signal, params, window_function, handle)
+    return (result["background"], result["integers"]) if return_periods else result["background"]
 
 
 def adaptive_f64(audio_signal, sampling_frequency, tunables, handle=None, return_periods=False):
     """repet.adaptive with the reference's calling convention (repet.py:422-568)."""
-    background, periods = _single_f64(
-        "repet_adaptive_f64", "adaptive", audio_signal, sampling_frequency, tunables, handle,
-        lambda params, number_samples: number_of_frames(number_samples, params.window_length, params.step_length),
-    )
-    return (background, periods) if return_periods else background
+    params, window_function = derive_params(sampling_frequency, tunables, "adaptive")
+    result = _run_f64("adaptive", audio_signal, params, window_function, handle)
+    return (result["background"], result["integers"]) if return_periods else result["background"]
 
 
 def driver_batch(driver, audio, sampling_frequency, tunables, handle=None):
     """original / extended / adaptive over a batch: audio (B, C, S) float32 planar host memory.
     Returns (background (B, C, S) float32, integer outputs (B, ints_per_clip) int32)."""
-    handle = handle or get_handle()
-    audio = np.ascontiguousarray(audio, dtype=np.float32)
-    if audio.ndim != 3:
-        raise ValueError("audio must have shape (clips, channels, samples)")
-    number_clips, number_channels, number_samples = audio.shape
-    params, _ = derive_params(sampling_frequency, tunables, driver)
     if driver not in METHODS:
         raise ValueError("unknown driver %r" % driver)
-    if needs_general_path(params, number_channels):
-        return _separate_batch_general(driver, audio, 0, 0, sampling_frequency, tunables, handle, None)
-    handle.ensure_window(params.window_length)
-    if driver == "original":
-        per_clip = 1
-    elif driver == "extended":
-        per_clip = handle.lib.repet_extended_segments(ctypes.byref(params), number_samples)
-    elif driver == "adaptive":
-        per_clip = number_of_frames(number_samples, params.window_length, params.step_length)
-    elif driver == "sim":
-        per_clip = number_of_frames(number_samples, params.window_length, params.step_length) * (params.similarity_number + 1)
-    elif driver == "simonline":
-        per_clip = max(0, handle.lib.repet_simonline_frames(ctypes.byref(params), number_samples)) * (
-            params.similarity_number + 1
-        )
-    else:
-        raise ValueError("unknown driver %r" % driver)
-    background = np.empty_like(audio)
-    ints = np.zeros((number_clips, max(1, per_clip)), dtype=np.int32)
-    try:
-        handle.check(
-            getattr(handle.lib, "repet_%s_batch" % driver)(
-                handle.h, _ptr(audio), number_clips, number_channels, number_samples, ctypes.byref(params), _ptr(background),
-                _ptr(ints),
-            )
-        )
-    except NotImplementedError:
-        return _separate_batch_general(driver, audio, 0, 0, sampling_frequency, tunables, handle, None)
-    return background, ints
-
-
-FORMATS = {"f32": 0, "pcm16": 1}  # REPET_FMT_F32_PLANAR, REPET_FMT_PCM16
+    params, window_function = derive_params(sampling_frequency, tunables, driver)
+    return _run_batch(driver, audio, params, window_function, handle)
 
 
 class PinnedArray:
@@ -842,80 +835,8 @@ def separate_batch(driver, audio, sampling_frequency, tunables, handle=None, in_
     one host thread per GPU over the same C entry point (clips are independent: no collective, SURVEY.md 8(e))."""
     if driver not in METHODS:
         raise ValueError("unknown driver %r" % driver)
-    in_code, out_code = FORMATS[in_format], FORMATS[out_format]
-    audio = np.ascontiguousarray(audio, dtype=np.int16 if in_code else np.float32)
-    if audio.ndim != 3:
-        raise ValueError("audio must have shape (clips, channels, samples) [f32] or (clips, samples, channels) [pcm16]")
-    if in_code:
-        number_clips, number_samples, number_channels = audio.shape
-    else:
-        number_clips, number_channels, number_samples = audio.shape
-    params, _ = derive_params(sampling_frequency, tunables, driver)
-    lib = load_library()
-    if needs_general_path(params, number_channels):
-        return _separate_batch_general(driver, audio, in_code, out_code, sampling_frequency, tunables, handle, out)
-    per_clip = int(lib.repet_ints_per_clip(METHODS[driver], ctypes.byref(params), number_samples))
-    out_shape = (number_clips, number_samples, number_channels) if out_code else (number_clips, number_channels, number_samples)
-    out_dtype = np.int16 if out_code else np.float32
-    if out is None:
-        out = np.empty(out_shape, dtype=out_dtype)
-    elif out.shape != out_shape or out.dtype != out_dtype or not out.flags.c_contiguous:
-        raise ValueError("out must be a C-contiguous %s array of shape %s" % (np.dtype(out_dtype).name, out_shape))
-    ints = np.zeros((number_clips, max(1, per_clip)), dtype=np.int32)
-
-    def run(h, first, stop):
-        if stop <= first:
-            return
-        h.ensure_window(params.window_length)
-        h.check(lib.repet_separate_batch(
-            h.h, METHODS[driver], _ptr(audio[first:stop]), in_code, stop - first, number_channels, number_samples,
-            ctypes.byref(params), _ptr(out[first:stop]), out_code, _ptr(ints[first:stop])))
-
-    if devices is None:
-        try:
-            run(handle or get_handle(), 0, number_clips)
-        except NotImplementedError:  # a shape or tunable the fast kernels refuse (e.g. a period range above 1024 frames)
-            return _separate_batch_general(driver, audio, in_code, out_code, sampling_frequency, tunables, handle, out)
-        return out, ints
-    devices = [int(d) for d in devices]
-    if not devices:
-        raise ValueError("devices must name at least one GPU")
-    handles = [get_handle(d) for d in devices]  # created on this thread: one handle per GPU
-    errors = []
-
-    def worker(h, first, stop):
-        try:
-            run(h, first, stop)
-        except BaseException as exc:  # re-raised on the caller's thread
-            errors.append(exc)
-
-    threads = [threading.Thread(target=worker, args=(h, lo, hi))
-               for h, (lo, hi) in zip(handles, shard_bounds(number_clips, len(devices)))]
-    for t in threads:
-        t.start()
-    for t in threads:
-        t.join()
-    if errors:
-        raise errors[0]
-    return out, ints
-
-
-def _separate_batch_general(driver, audio, in_code, out_code, sampling_frequency, tunables, handle, out):
-    """separate_batch for inputs outside the fast kernels' shapes: clip by clip on the general float64 path."""
-    backgrounds, integers = [], []
-    for clip in audio:
-        x = clip.astype(np.float64) / 32768.0 if in_code else clip.T.astype(np.float64)  # repet.py:929
-        y, ints = general_f64(driver, x, sampling_frequency, tunables, handle=handle)
-        if out_code:
-            backgrounds.append(np.clip(np.rint(y.astype(np.float32) * np.float32(32768.0)), -32768, 32767).astype(np.int16))
-        else:
-            backgrounds.append(np.ascontiguousarray(y.T.astype(np.float32)))
-        integers.append(ints)
-    result = np.stack(backgrounds) if backgrounds else np.zeros((0,) + audio.shape[1:], np.int16 if out_code else np.float32)
-    if out is not None:
-        out[...] = result
-        result = out
-    return result, np.stack(integers) if integers else np.zeros((0, 1), np.int32)
+    params, window_function = derive_params(sampling_frequency, tunables, driver)
+    return _run_batch(driver, audio, params, window_function, handle, in_format, out_format, out, devices)
 
 
 # ------------------------------------------------------------------------------------------
@@ -997,8 +918,8 @@ def sharded_track(driver, audio_signal, sampling_frequency, tunables, devices):
     separated with a halo that covers the beat-spectrogram segments and the median taps of its frames, and only
     its own samples are kept), bit for bit for `simonline` (each block replays its similarity history)."""
     x = np.ascontiguousarray(audio_signal, dtype=np.float64)
-    number_samples, number_channels = x.shape
-    params, _ = derive_params(sampling_frequency, tunables, driver)
+    number_samples, _ = x.shape
+    params, window_function = derive_params(sampling_frequency, tunables, driver)
     blocks = track_time_blocks(driver, number_samples, params, len(list(devices)))
     if len(blocks) == 1:
         return {"extended": extended_f64, "adaptive": adaptive_f64, "simonline": simonline_f64}[driver](
@@ -1046,20 +967,9 @@ def sharded_track(driver, audio_signal, sampling_frequency, tunables, devices):
         # frames that touch [a, b): up to the one starting below b; the window must hold whole frames
         last_frame = min((b - 1) // H, max(0, -(-(number_samples - N) // H)))
         hi = min(number_samples, last_frame * H + N)
-        window = np.ascontiguousarray(x[lo:hi])
-        p = RepetParams()
-        ctypes.memmove(ctypes.byref(p), ctypes.byref(params), ctypes.sizeof(RepetParams))
+        p = RepetParams.from_buffer_copy(params)
         p.online_frame_base = int(first_frame)
-        y = np.empty_like(window)
-        if needs_general_path(p, number_channels):
-            hamming = np.ascontiguousarray(hamming_window(N), dtype=np.float64)
-            h.check(h.lib.repet_general_f64(h.h, METHODS["simonline"], _ptr(window), window.shape[0], number_channels,
-                                            ctypes.byref(p), _ptr(hamming), _ptr(y), None, 0))
-        else:
-            h.ensure_window(N)
-            h.check(h.lib.repet_simonline_f64(h.h, _ptr(window), window.shape[0], number_channels, ctypes.byref(p), _ptr(y),
-                                              None, 0))
-        return y[a - lo : b - lo]
+        return _run_f64("simonline", x[lo:hi], p, window_function, h)["background"][a - lo : b - lo]
 
     jobs = [(lambda h, a=a, b=b: online_block(h, a, b)) for a, b in blocks]
     for (a, b), y in zip(blocks, _run_shards(jobs, devices)):
@@ -1160,36 +1070,23 @@ def unpack_lists(ints, number_frames, number):
 
 def sim_f64(audio_signal, sampling_frequency, tunables, handle=None, return_indices=False):
     """repet.sim with the reference's calling convention (repet.py:571-709)."""
-    number = int(tunables["similarity_number"])
-    frames = {}
-
-    def capacity(params, number_samples):
-        frames["T"] = number_of_frames(number_samples, params.window_length, params.step_length)
-        return frames["T"] * (number + 1)
-
-    background, ints = _single_f64("repet_sim_f64", "sim", audio_signal, sampling_frequency, tunables, handle, capacity)
+    params, window_function = derive_params(sampling_frequency, tunables, "sim")
+    result = _run_f64("sim", audio_signal, params, window_function, handle)
     if return_indices:
-        return background, unpack_lists(ints, frames["T"], number)
-    return background
+        ints, number = result["integers"], params.similarity_number
+        return result["background"], unpack_lists(ints, len(ints) // (number + 1), number)
+    return result["background"]
 
 
 def simonline_f64(audio_signal, sampling_frequency, tunables, handle=None, return_indices=False):
     """repet.simonline with the reference's calling convention (repet.py:712-911).  With
     return_indices the lists of frames >= buffer_frames-1 hold FRAME indices (most similar first)."""
-    lib = load_library()
-    number = int(tunables["similarity_number"])
-    frames = {}
-
-    def capacity(params, number_samples):
-        frames["T"] = max(0, lib.repet_simonline_frames(ctypes.byref(params), number_samples))
-        return frames["T"] * (number + 1)
-
-    background, ints = _single_f64(
-        "repet_simonline_f64", "simonline", audio_signal, sampling_frequency, tunables, handle, capacity
-    )
+    params, window_function = derive_params(sampling_frequency, tunables, "simonline")
+    result = _run_f64("simonline", audio_signal, params, window_function, handle)
     if return_indices:
-        return background, unpack_lists(ints, frames["T"], number)
-    return background
+        ints, number = result["integers"], params.similarity_number
+        return result["background"], unpack_lists(ints, len(ints) // (number + 1), number)
+    return result["background"]
 
 
 def selfsimilarity(data_matrix, handle=None):
@@ -1273,22 +1170,9 @@ def acorr(data_matrix, handle=None):
 def original_batch_pcm16(pcm, sampling_frequency, tunables, handle=None):
     """`original` over int16 PCM clips in WAV order: pcm (B, S, C) int16 -> (background (B, C, S) float32,
     periods (B,) int32).  The samples are normalised by 2^15 on the device, as repet.wavread does."""
-    handle = handle or get_handle()
-    pcm = np.ascontiguousarray(pcm, dtype=np.int16)
-    if pcm.ndim != 3:
-        raise ValueError("pcm must have shape (clips, samples, channels)")
-    number_clips, number_samples, number_channels = pcm.shape
-    params, _ = derive_params(sampling_frequency, tunables)
-    handle.ensure_window(params.window_length)
-    background = np.empty((number_clips, number_channels, number_samples), dtype=np.float32)
-    periods = np.zeros(number_clips, dtype=np.int32)
-    handle.check(
-        handle.lib.repet_original_batch_pcm16(
-            handle.h, _ptr(pcm), number_clips, number_channels, number_samples, ctypes.byref(params), _ptr(background),
-            _ptr(periods),
-        )
-    )
-    return background, periods
+    params, window_function = derive_params(sampling_frequency, tunables)
+    background, ints = _run_batch("original", pcm, params, window_function, handle, in_format="pcm16")
+    return background, ints[:, 0]
 
 
 class SimOnlineStreamHost:
@@ -1309,7 +1193,7 @@ class SimOnlineStreamHost:
         self.fs = sampling_frequency
         self.channels = int(number_channels)
         self.tunables = dict(tunables)
-        self.params, _ = derive_params(sampling_frequency, self.tunables, "simonline")
+        self.params, self.window_function = derive_params(sampling_frequency, self.tunables, "simonline")
         self.N, self.H, self.B = self.params.window_length, self.params.step_length, self.params.buffer_frames
         self.buffer = np.zeros((0, self.channels), dtype=np.float64)  # samples from frame `buffer_frame0` on
         self.buffer_frame0 = 0
@@ -1319,27 +1203,10 @@ class SimOnlineStreamHost:
     def _run_window(self, first_frame, number_samples):
         """simonline on buffer samples [first_frame*H - buffer_frame0*H, ... + number_samples)."""
         lo = (first_frame - self.buffer_frame0) * self.H
-        window = np.ascontiguousarray(self.buffer[lo : lo + number_samples])
-        params = RepetParams()
-        ctypes.memmove(ctypes.byref(params), ctypes.byref(self.params), ctypes.sizeof(RepetParams))
+        params = RepetParams.from_buffer_copy(self.params)
         params.online_frame_base = int(first_frame)
-        out = np.empty_like(window)
-        if needs_general_path(params, self.channels):
-            hamming = np.ascontiguousarray(hamming_window(params.window_length), dtype=np.float64)
-            self.handle.check(
-                self.handle.lib.repet_general_f64(
-                    self.handle.h, METHODS["simonline"], _ptr(window), window.shape[0], self.channels, ctypes.byref(params),
-                    _ptr(hamming), _ptr(out), None, 0
-                )
-            )
-            return out
-        self.handle.ensure_window(params.window_length)
-        self.handle.check(
-            self.handle.lib.repet_simonline_f64(
-                self.handle.h, _ptr(window), window.shape[0], self.channels, ctypes.byref(params), _ptr(out), None, 0
-            )
-        )
-        return out
+        return _run_f64("simonline", self.buffer[lo : lo + number_samples], params, self.window_function,
+                        self.handle)["background"]
 
     def _advance(self, final_until, total_samples_for_window):
         """Emit background samples [emitted, final_until)."""

@@ -245,3 +245,55 @@ def test_batches_fall_back_to_the_general_path_when_the_fast_kernels_refuse(repe
         y_ref, det = oracle.original(audio[i].T.astype(np.float64), FS, return_details=True, period_range=(1, 29))
         assert int(periods[i]) == det["period"]
         _signal_close(background[i].T.astype(np.float64), y_ref, "clip %d" % i, tol=1e-6)
+
+
+def test_separate_falls_back_to_the_general_path_when_the_fast_kernels_refuse(repet):
+    """`repet.separate` with a period range above 1024 frames: the background, foreground, period and spectrograms
+    come from the general path."""
+    x = repet_synth.make_batch(995, 1, 90 * FS)[0].T.astype(np.float64)
+    saved = repet.period_range
+    try:
+        repet.period_range = [1, 29]  # 1249 frames
+        parts = repet.separate(x, FS)
+    finally:
+        repet.period_range = saved
+    y_ref, det = oracle.original(x, FS, return_details=True, period_range=(1, 29))
+    assert parts["integers"].dtype == np.int32 and list(parts["integers"]) == [det["period"]]
+    _signal_close(parts["background"], y_ref, "background")
+    _signal_close(parts["foreground"], x - y_ref, "foreground", tol=1e-8)
+    N, w, H = oracle.stft_parameters(FS)
+    for name, signal in (("audio_spectrogram", x), ("background_spectrogram", y_ref), ("foreground_spectrogram", x - y_ref)):
+        assert parts[name].dtype == np.float64
+        _signal_close(parts[name], np.abs(oracle.stft(np.mean(signal, axis=1), w, H)[: N // 2 + 1]), name, tol=1e-8)
+
+
+def test_sharded_batch_falls_back_to_the_general_path_when_the_fast_kernels_refuse(repet):
+    """`separate_batch(devices=[0])` with a period range above 1024 frames: the shard's refusal sends the batch to
+    the general path."""
+    audio = repet_synth.make_batch(995, 2, 90 * FS)
+    saved = repet.period_range
+    try:
+        repet.period_range = [1, 29]
+        background, ints = repet.separate_batch(audio, FS, "original", devices=[0])
+    finally:
+        repet.period_range = saved
+    assert background.shape == audio.shape and background.dtype == np.float32 and ints.shape == (2, 1)
+    for i in range(2):
+        y_ref, det = oracle.original(audio[i].T.astype(np.float64), FS, return_details=True, period_range=(1, 29))
+        assert int(ints[i, 0]) == det["period"]
+        _signal_close(background[i].T.astype(np.float64), y_ref, "clip %d" % i, tol=1e-6)
+
+
+@pytest.mark.parametrize("fs,channels", [(96000, 2), (FS, 3)])
+def test_pcm16_batch_takes_the_general_path(repet, fs, channels):
+    """`original_batch_pcm16` at 96 kHz and with three channels: shapes the fast kernels are not compiled for."""
+    audio = repet_synth.make_batch(1000 + channels, 2, 8 * fs, channels, fs, step_length=2048 if fs > FS else 1024)
+    pcm = np.clip(np.rint(np.transpose(audio, (0, 2, 1)) * 32768.0), -32768, 32767).astype(np.int16)
+    background, periods = repet.original_batch_pcm16(pcm, fs)
+    assert background.shape == audio.shape and background.dtype == np.float32
+    assert periods.shape == (2,) and periods.dtype == np.int32
+    for i in range(2):
+        y_ref, det = oracle.original(pcm[i] / 32768.0, fs, return_details=True)
+        assert int(periods[i]) == det["period"]
+        _signal_close(background[i].T.astype(np.float64), y_ref, "%d Hz, %d channels, clip %d" % (fs, channels, i),
+                      tol=1e-6)
